@@ -393,7 +393,7 @@ def run_config3(args, pkg):
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a B200: the matching path has no CPU fallback")
     total = args.pairs or 100_000_000
-    blk = config3_block(args, pkg, total, min(total, 10_000_000), steps=max(1, min(args.steps, 3)))
+    blk = config3_block(args, pkg, total, min(total, 10_000_000), steps=args.steps)
     live = blk["shapes"][0]["score_only"]
     emit({"metric": METRIC, "value": live["M_pairs_per_min"], "unit": "M read/window pairs per min (SW microbench, 150 x 150, score + coordinates)",
           "n_gpus": 1, "steps": args.steps, "warmup": args.warmup, "ms_per_step": live["ms"], "higher_is_better": True, "scaling": "weak",
@@ -712,14 +712,20 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=0, help="pairs for the cpu_baseline leg (rank 0, N=1; 0 = per workload)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="default workload only: skip the config1 / config3 / config5 / cli blocks")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy (config1 / config2 / config4)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "kslam" or args.workload not in DEFAULT_PAIRS):
+        raise SystemExit("--dump-outputs: only the matching-path workloads (config1, config2, config4) write their outputs")
 
     pkg = ge.load_pkg()
     if args.workload == "config3":
         return run_config3(args, pkg)
     if args.workload == "config5":
-        blk = config5_block(args, pkg, 10, args.pairs or 10_000_000)
-        return emit({"metric": METRIC, "value": blk["value"], "unit": UNIT, "n_gpus": 1, "steps": 10, "warmup": 0, "ms_per_step": blk["wall_s"] * 100,
+        blk = config5_block(args, pkg, args.steps, args.pairs or 10_000_000)
+        return emit({"metric": METRIC, "value": blk["value"], "unit": UNIT, "n_gpus": 1, "steps": args.steps, "warmup": 0,
+                     "ms_per_step": blk["wall_s"] / args.steps * 1e3,
                      "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "int16x2 (SW) / u64 (k-mers) / f64 (MAPQ)", "data": "synthetic",
                      "config": {"workload": blk["workload"]}, **{k: v for k, v in blk.items() if k not in ("value", "unit", "workload")}})
     if args.workload == "sam":
@@ -801,6 +807,8 @@ def main():
     t_res = tw1 - tw0                           # library calls are synchronous: wall == device time of the chain
     tm = al.timings()
     launches = (tm["kernel_launches"] - launches0) // max(1, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, al.fetch_pairs(copy=False))
 
     # ---- e2e: host buffers in, results back on the host ------------------------------------------
     # The reference-facing call with HOST buffers: kslam_align_pair_batch = the body of the batch loop (SLAM.h:209-214),
@@ -984,6 +992,33 @@ def e2e_pipeline(ctxs, rb, ro, n_batches, device, compact, last):
     [t.start() for t in th]; [t.join() for t in th]
     if errs:
         raise errs[0]
+
+
+def dump_outputs(out_dir, res, seed=0, limit=60 << 20):
+    """--dump-outputs DIR: what kslam_fetch_pairs hands the caller after the last timed step (pair-sorted overlaps, their
+    CIGARs, pair records), one float64 .npy per field (all are 32-bit integers, exact in float64), so that two builds can
+    be compared output for output on the same seeded workload. Larger outputs are cut to a seeded sample of rows, the
+    same rows for the same record counts: 2^17 overlaps and 2^18 pairs. cigar_off, a position in this build's CIGAR pool,
+    is given as the words it points to: cigar_words holds the whole CIGARs (cigar_len words each) of the sampled overlaps
+    in order, as many as fit in `limit` bytes of arrays in all (every one of them unless the sample averages more than
+    ~35 words per CIGAR). A workload without CIGARs (config2, config4) has no cigar_words."""
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(seed)
+
+    def sample(a, k):
+        return a if len(a) <= k else a[np.sort(rng.choice(len(a), k, replace=False))]
+    ov, pr = sample(res.sorted_overlaps, 1 << 17), sample(res.pairs, 1 << 18)
+    arrays = {"counts": [len(res.sorted_overlaps), len(res.pairs)]}
+    arrays.update({"sorted_overlaps_" + f: ov[f] for f in ov.dtype.names if f != "cigar_off"})
+    arrays.update({"pairs_" + f: pr[f] for f in pr.dtype.names if f != "pad"})
+    if len(res.cigar_pool):
+        room = (limit - 8 * sum(np.size(a) for a in arrays.values())) // 8          # float64 words left
+        k = int(np.searchsorted(np.cumsum(ov["cigar_len"], dtype=np.int64), room, side="right"))
+        arrays["cigar_words"] = np.concatenate([res.cigar_pool[o:o + n] for o, n in zip(ov["cigar_off"][:k], ov["cigar_len"][:k])])
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+    n_cig = f", CIGARs of the first {k}" if "cigar_words" in arrays else ""
+    log(f"[bench] wrote {len(arrays)} arrays ({len(ov)} of {len(res.sorted_overlaps)} overlaps{n_cig}, {len(pr)} of {len(res.pairs)} pairs) to {out_dir}")
 
 
 def d2h_bytes(res, compact):

@@ -7,6 +7,7 @@ machines where the reference sources are absent. Inputs are seeded (k-slam_b200/
 """
 import os
 import sys
+import zipfile
 
 import numpy as np
 
@@ -15,6 +16,15 @@ sys.path.insert(0, os.path.dirname(HERE))
 import _lib as T  # noqa: E402
 
 synth = T.load_pkg().synth
+
+
+def savez_lzma(path, **arrays):
+    """np.savez_compressed with LZMA members instead of deflate (np.load reads both): the k-mer lists of the pipeline
+    fixtures compress to well under the 1 MB a stored file may take."""
+    with zipfile.ZipFile(path, "w", zipfile.ZIP_LZMA) as z:
+        for k, a in arrays.items():
+            with z.open(k + ".npy", "w", force_zip64=True) as f:
+                np.lib.format.write_array(f, np.asanyarray(a), allow_pickle=False)
 
 
 def pipeline_fixture(name, gb, go, rb, ro, params):
@@ -27,7 +37,7 @@ def pipeline_fixture(name, gb, go, rb, ro, params):
     seeds = R.seeds(raw=False)
     ov, pool = R.align_to_database()
     ovs, pools, pairs = R.screen_and_pair()
-    np.savez_compressed(
+    savez_lzma(
         os.path.join(HERE, name), gen_bases=gb, gen_offs=go, read_bases=rb, read_offs=ro,
         params=np.array([params.match, params.mismatch, params.gap_open, params.gap_extend,
                          params.score_threshold, params.report_cigar], dtype=np.int64),
@@ -71,6 +81,27 @@ def sam_fixture(name):
     R = T.Ref(gb, go, rb[:0], ro[:1], T.default_params()); hdr = T.ref_sam_header(R, "SLAM golden"); R.close()
     np.savez_compressed(os.path.join(HERE, name), gb=gb, go=go, rb=rb, ro=ro, quals=quals, ids=idb, id_offs=ido, ov=ov, pool=pool, pairs=pairs,
                         sam=np.frombuffer(text, np.uint8), max_insert=mi, header=np.frombuffer(hdr, np.uint8))
+
+
+def sam_digest_fixture(name):
+    """Digest of the reference's SAM text (SLAM.h:215-239 chain + SAM.h) for a 6000-pair batch, too large to store at
+    > 1 MB. test_sam_host.py feeds the library the oracle's alignments for this batch, so they are checked here against
+    the reference's (every overlap field but cigar_off, the CIGARs, the pairs) before the text is digested.
+    The file in the repository was NOT made by this function: it was recorded where the reference sources were absent,
+    from the library's SAM writer on the oracle's alignments, with sam.cu as it stood when test_sam_host.py last compared
+    this batch (on the reference's alignments) with the reference's text. Nothing in the repository shows that the two
+    agree on this batch; on the 300-pair batch of the same genomes they do (sam_config1_mini.npz). Running this function
+    where the reference exists settles it: the same arrays mean the digest is the reference's."""
+    from test_sam_host import crc32_of, make_inputs, oracle_side, reference_side, sam_digest
+    gb, go, rb, ro, quals, idb, ido = make_inputs(T.load_pkg(), 5, n_pairs=6000, kind="random")
+    ov, pool, pairs = oracle_side(gb, go, rb, ro)
+    rov, rpool, rpairs, text, mi, _ = reference_side(gb, go, rb, ro, quals, 1)
+    assert len(ov) == len(rov) and all(np.array_equal(ov[f], rov[f]) for f in ov.dtype.names if f != "cigar_off"), "overlaps"
+    assert T.cigars_of(ov, pool) == T.cigars_of(rov, rpool), "cigars"
+    assert np.array_equal(pairs, rpairs), "pairs"
+    np.savez_compressed(os.path.join(HERE, name), max_insert=mi, inputs_crc32=crc32_of(gb, go, rb, ro, quals, idb, ido),
+                        alignments_crc32=crc32_of(ov, pool, pairs), **sam_digest(text))
+    print(name, "sam bytes", len(text), "lines", text.count(b"\n"))
 
 
 def meta_fixture(name):
@@ -138,6 +169,8 @@ def main():
         return meta_fixture("meta_mini.npz")
     if len(sys.argv) > 1 and sys.argv[1] == "boost":
         return boost_archive_fixture("database_boost178.npz")
+    if len(sys.argv) > 1 and sys.argv[1] == "sam-digest":
+        return sam_digest_fixture("sam_random_6000_digest.npz")
     boost_archive_fixture("database_boost178.npz")
     meta_fixture("meta_mini.npz")
     fastq_fixture("fastq_reader.npz")
