@@ -41,7 +41,7 @@ __device__ __forceinline__ uint32_t rs2_digit_peers(uint32_t d) {
 __device__ __forceinline__ uint32_t rs2_look_back(volatile uint32_t *state, uint32_t tile, uint32_t d, uint32_t count) {
   volatile uint32_t *mine = state + (size_t)tile * 256 + d;
   uint32_t excl = 0;
-  int64_t t = (int64_t)tile - 1;
+  int32_t t = (int32_t)tile - 1;
   while (t >= 0) {
     uint32_t s[8];
 #pragma unroll
@@ -69,56 +69,6 @@ __device__ __forceinline__ uint32_t rs2_look_back(volatile uint32_t *state, uint
   return excl;
 }
 
-// Two-level look-back (an experiment, off by default: KSLAM_RS_LB=1; it measured 4 % slower than the flat walk, so the
-// chain of predecessor loads is not what bounds a tile). With ~300 tiles in flight the flat walk above sums up to a few hundred predecessor aggregates,
-// eight loads per round trip to L2, and that chain — not the bytes — sets the life time of a tile (the pass sat at 0.53
-// of the copy peak). Tiles are grouped by RS2_GROUP: a tile sums the aggregates of the predecessors of ITS group (at most
-// 15: two rounds), the last tile of a group publishes the group's total as soon as it has that sum, and everybody then
-// walks the group totals (300 / 16 in flight: three rounds). An inclusive prefix met on either level ends the walk.
-// Entries beyond the range of a level read as a published aggregate of 0, which keeps the eight-at-a-time fast path.
-#define RS2_GROUP 16
-__device__ __forceinline__ bool rs2_walk(volatile uint32_t *base, int32_t &t, int32_t lo, uint32_t &excl) {
-  while (t >= lo) {
-    uint32_t s[8];
-#pragma unroll
-    for (int k = 0; k < 8; k++) s[k] = (t - k >= lo) ? base[(size_t)(t - k) * 256] : RS2_AGG;
-    const uint32_t all = s[0] & s[1] & s[2] & s[3] & s[4] & s[5] & s[6] & s[7];
-    const uint32_t any = s[0] | s[1] | s[2] | s[3] | s[4] | s[5] | s[6] | s[7];
-    if ((all & RS2_AGG) && !(any & RS2_INCL)) {
-      excl += s[0] + s[1] + s[2] + s[3] + s[4] + s[5] + s[6] + s[7];
-      t -= 8;
-      continue;
-    }
-    bool done = false;
-    int used = 0;
-#pragma unroll
-    for (int k = 0; k < 8; k++) {
-      if (!done && used == k && (s[k] & (RS2_AGG | RS2_INCL))) {
-        excl += s[k] & RS2_VAL; used = k + 1;
-        if (s[k] & RS2_INCL) done = true;
-      }
-    }
-    if (done) return true;
-    t -= used;                                             // an unpublished predecessor: fetch again from there
-  }
-  return false;
-}
-__device__ __forceinline__ uint32_t rs2_look_back2(volatile uint32_t *state, volatile uint32_t *gstate, uint32_t tile, uint32_t d, uint32_t count) {
-  const uint32_t g = tile / RS2_GROUP;
-  const bool closes = tile % RS2_GROUP == RS2_GROUP - 1;    // the last tile of its group
-  uint32_t excl = 0;
-  int32_t t = (int32_t)tile - 1;
-  bool absolute = rs2_walk(state + d, t, (int32_t)(g * RS2_GROUP), excl);
-  if (!absolute) {
-    if (closes) gstate[(size_t)g * 256 + d] = RS2_AGG | (excl + count);      // the group's total: the groups behind can move on
-    int32_t gg = (int32_t)g - 1;
-    rs2_walk(gstate + d, gg, 0, excl);
-  }
-  state[(size_t)tile * 256 + d] = RS2_INCL | (excl + count);
-  if (closes) gstate[(size_t)g * 256 + d] = RS2_INCL | (excl + count);
-  return excl;
-}
-
 // REC = Rec16: 16-byte records sorted by .key (WORD 0) or .val (WORD 1); REC = uint64_t: bare 8-byte keys (half the bytes
 // per record and pass: the packed seeds of join.cu, WORD ignored).
 template <int RS_THREADS, int RS_IPT, int WORD, typename REC>
@@ -126,12 +76,11 @@ __global__ void __launch_bounds__(RS_THREADS, 2)
 k_rs_pass2(const REC *__restrict__ in, REC *__restrict__ out, uint64_t n, uint32_t shift, uint32_t mask,
            const unsigned long long *__restrict__ digit_base,  // [256] exclusive global offsets
            volatile uint32_t *state,                           // [tiles][256], zero-initialised
-           volatile uint32_t *gstate,                          // [tiles / RS2_GROUP][256], zero-initialised; nullptr: flat look-back
            uint32_t *__restrict__ ticket) {
   constexpr int RS_WARPS = RS_THREADS / 32;
   constexpr uint32_t RS_TILE = RS_THREADS * RS_IPT;
   static_assert(RS_THREADS >= 256 && RS_THREADS % 256 == 0, "threads 0..255 own one digit each");
-  extern __shared__ __align__(16) unsigned char smem_raw[];
+  extern __shared__ __align__(128) unsigned char smem_raw[];
   constexpr bool BARE = sizeof(REC) == 8;
   REC *stage = reinterpret_cast<REC *>(smem_raw);                                   // RS_TILE records
   uint32_t *whist = reinterpret_cast<uint32_t *>(smem_raw + RS_TILE * sizeof(REC)); // [RS_WARPS][256]
@@ -212,7 +161,7 @@ k_rs_pass2(const REC *__restrict__ in, REC *__restrict__ out, uint64_t n, uint32
 #pragma unroll
     for (int w = 0; w < 8; w++) if (w < (int)warp) wexcl += s_scan[w];
     const uint32_t dexcl = wexcl + inc - cnt_d;           // first position of digit `tid` in the staged tile
-    const uint32_t excl = tile ? (gstate ? rs2_look_back2(state, gstate, tile, tid, real_d) : rs2_look_back(state, tile, tid, real_d)) : 0u;
+    const uint32_t excl = tile ? rs2_look_back(state, tile, tid, real_d) : 0u;
     s_delta[tid] = digit_base[tid] + excl - dexcl;        // staged position j of this digit -> global position s_delta + j
 #pragma unroll
     for (int w = 0; w < RS_WARPS; w++) whist[w * 256 + tid] += dexcl;

@@ -11,7 +11,6 @@
 //
 // Roofline: HBM. Algorithmic bytes per record = 32 B x passes (+16 B for the histogram read).
 #include "common.cuh"
-#include <stdlib.h>
 
 #define RS_MAX_PASSES 8
 
@@ -71,8 +70,7 @@ k_rs_scan_hist(unsigned long long *__restrict__ ghist, uint32_t n_passes, uint64
 // lanes of the warp holding the same 8-bit digit. MATCH.ANY walks the distinct values of the warp one by one (32 of them
 // for random digits: the ADU pipe was the limiter of those passes, profiles/r1k); eight ballots cost the same for any
 // distribution.
-template <bool BALLOT> __device__ __forceinline__ uint32_t digit_peers(uint32_t d) {
-  if (!BALLOT) return __match_any_sync(0xffffffffu, d);
+__device__ __forceinline__ uint32_t digit_peers(uint32_t d) {
   uint32_t peers = 0xffffffffu;
 #pragma unroll
   for (int b = 0; b < 8; b++) {
@@ -116,7 +114,7 @@ __device__ __forceinline__ unsigned long long publish_and_look_back(volatile uns
 }
 
 // ---- one LSD pass ------------------------------------------------------------------------------
-template <int RS_THREADS, int RS_IPT, bool BALLOT>
+template <int RS_THREADS, int RS_IPT>
 __global__ void __launch_bounds__(RS_THREADS, (RS_THREADS * RS_IPT > 4096 ? 1 : (RS_THREADS * RS_IPT > 3072 ? 2 : (RS_THREADS * RS_IPT > 2048 ? 3 : 4))))
 k_rs_onesweep(const Rec16 *__restrict__ in, Rec16 *__restrict__ out, uint64_t n, uint32_t shift, uint32_t mask,
               uint32_t word,                                       // 0: sort by .key, 1: sort by .val
@@ -125,7 +123,7 @@ k_rs_onesweep(const Rec16 *__restrict__ in, Rec16 *__restrict__ out, uint64_t n,
               uint32_t *__restrict__ ticket) {
   constexpr int RS_WARPS = RS_THREADS / 32;
   constexpr uint32_t RS_TILE = RS_THREADS * RS_IPT;     // records per tile, staged in shared memory
-  extern __shared__ __align__(16) unsigned char smem_raw[];
+  extern __shared__ __align__(128) unsigned char smem_raw[];
   Rec16 *stage = reinterpret_cast<Rec16 *>(smem_raw);                               // RS_TILE records
   uint32_t *whist = reinterpret_cast<uint32_t *>(smem_raw + RS_TILE * sizeof(Rec16)); // [RS_WARPS][256]
   __shared__ uint32_t s_dexcl[256];
@@ -162,7 +160,7 @@ k_rs_onesweep(const Rec16 *__restrict__ in, Rec16 *__restrict__ out, uint64_t n,
   for (int i = 0; i < RS_IPT; i++) {
     const uint32_t idx = wbase + i * 32 + lane;
     const uint32_t d = idx < count ? ((uint32_t)((word ? val[i] : key[i]) >> shift) & mask) : 255u;
-    const uint32_t peers = digit_peers<BALLOT>(d);
+    const uint32_t peers = digit_peers(d);
     const uint32_t old = myhist[d];              // every peer reads the warp's running count (broadcast)
     __syncwarp();
     if ((peers & lt_mask) == 0) myhist[d] = old + __popc(peers);   // lowest peer publishes the new count
@@ -221,16 +219,7 @@ k_rs_onesweep(const Rec16 *__restrict__ in, Rec16 *__restrict__ out, uint64_t n,
   }
 }
 
-// ---- one LSD pass, persistent form: tiles arrive by bulk copy (TMA) while the previous one is processed ---------
-// k_rs_onesweep above loads a tile into 32 registers per thread, ranks it, stages it and writes it out, one phase after
-// the other; at 128 registers + 72 KB only two CTAs share an SM and ncu shows the memory pipe idle while they rank
-// (24 % warps active, 0.23 eligible warps per cycle, dram at 30 % of peak although the traffic is exactly the algorithmic
-// 32 B per record). Here a CTA stays resident and takes tiles from the ticket counter; one thread starts the bulk copy
-// (cp.async.bulk -> mbarrier, SASS UBLKCP) of tile t+1 into the second arrival buffer as soon as it has the ticket, so
-// the copy runs under the ranking / look-back / scatter / write-out of tile t. Records are ranked FROM shared memory
-// (LDS.128, the digit and the 16-bit rank are all a thread keeps: no key / value register arrays), scattered into a
-// third buffer in digit order and written out in contiguous runs. Tickets are handed out in order, so every predecessor
-// a look-back waits for belongs to a CTA that is already running: no deadlock.
+// mbarrier + bulk copy (cp.async.bulk, SASS UBLKCP) helpers: k_rs_pass2 loads its tile with one bulk copy
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
@@ -252,149 +241,9 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
 
 #include "radix_pass2.cuh"
 
-template <int RS_THREADS, int RS_IPT, int CTAS_PER_SM>
-__global__ void __launch_bounds__(RS_THREADS, CTAS_PER_SM)
-k_rs_sweep_tma(const Rec16 *__restrict__ in, Rec16 *__restrict__ out, uint64_t n, uint32_t shift, uint32_t mask,
-               uint32_t word,                                       // 0: sort by .key, 1: sort by .val
-               const unsigned long long *__restrict__ digit_base,  // [256] exclusive global offsets
-               volatile unsigned long long *tile_state,            // [tiles][256], zero-initialised
-               uint32_t *__restrict__ ticket, uint32_t n_tiles) {
-  constexpr int RS_WARPS = RS_THREADS / 32;
-  constexpr uint32_t RS_TILE = RS_THREADS * RS_IPT;
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  Rec16 *arrive0 = reinterpret_cast<Rec16 *>(smem_raw), *arrive1 = arrive0 + RS_TILE, *stage = arrive1 + RS_TILE;
-  uint32_t *whist = reinterpret_cast<uint32_t *>(stage + RS_TILE);   // [RS_WARPS][256]
-  __shared__ uint32_t s_dexcl[256];
-  __shared__ unsigned long long s_gbase[256];
-  __shared__ uint32_t s_scan[32];
-  __shared__ uint32_t s_tile[2];
-  __shared__ __align__(8) uint64_t s_bar[2];
-
-  const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  auto start_copy = [&](uint32_t t, uint32_t slot) {       // one thread: arm the barrier, start the bulk copy of tile t
-    const uint64_t base = (uint64_t)t * RS_TILE;
-    const uint32_t cnt = (uint32_t)((n - base) < RS_TILE ? (n - base) : RS_TILE);
-    mbar_expect_tx(&s_bar[slot], cnt * (uint32_t)sizeof(Rec16));
-    bulk_load(slot ? arrive1 : arrive0, in + base, cnt * (uint32_t)sizeof(Rec16), &s_bar[slot]);
-  };
-  if (tid == 0) {
-    mbar_init(&s_bar[0], 1); mbar_init(&s_bar[1], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    const uint32_t t = atomicAdd(ticket, 1u);
-    s_tile[0] = t;
-    if (t < n_tiles) start_copy(t, 0);
-  }
-  __syncthreads();
-
-  const uint32_t wbase = warp * 32 * RS_IPT;
-  const uint32_t lt_mask = (1u << lane) - 1;
-  uint32_t *myhist = whist + warp * 256;
-  uint32_t parity0 = 0, parity1 = 0;
-  for (uint32_t slot = 0;; slot ^= 1) {
-    const uint32_t tile = s_tile[slot];
-    if (tile >= n_tiles) break;
-    const Rec16 *arr = slot ? arrive1 : arrive0;
-    if (tid == 0) {                                        // next ticket, its copy goes into the other arrival buffer
-      const uint32_t t = atomicAdd(ticket, 1u);
-      s_tile[slot ^ 1] = t;
-      if (t < n_tiles) start_copy(t, slot ^ 1);
-    }
-#pragma unroll
-    for (uint32_t i = tid; i < RS_WARPS * 256; i += RS_THREADS) whist[i] = 0;
-    __syncthreads();                                       // histograms clear; the previous tile's write-out is over
-    const uint64_t tile_base = (uint64_t)tile * RS_TILE;
-    const uint32_t count = (uint32_t)((n - tile_base) < RS_TILE ? (n - tile_base) : RS_TILE);
-    mbar_wait(&s_bar[slot], slot ? parity1 : parity0);
-    if (slot) parity1 ^= 1; else parity0 ^= 1;
-
-    // 1. per-warp digit ranks, records read from the arrival buffer; (warp, item, lane) order == input order (stability)
-    uint32_t dr[RS_IPT];                                   // digit << 16 | rank inside (warp, digit)
-#pragma unroll
-    for (int i = 0; i < RS_IPT; i++) {
-      const uint32_t idx = wbase + i * 32 + lane;
-      uint32_t d = 255u;                                   // padding sorts to the very end of the tile
-      if (idx < count) {
-        const ulonglong2 r = *reinterpret_cast<const ulonglong2 *>(arr + idx);
-        d = (uint32_t)((word ? r.y : r.x) >> shift) & mask;
-      }
-      const uint32_t peers = digit_peers<true>(d);
-      const uint32_t old = myhist[d];
-      __syncwarp();
-      if ((peers & lt_mask) == 0) myhist[d] = old + __popc(peers);
-      __syncwarp();
-      dr[i] = (d << 16) | (old + __popc(peers & lt_mask));
-    }
-    __syncthreads();
-
-    // 2. thread d (< 256) owns digit d: exclusive offsets over warps, tile count, publish + look back, tile-local scan
-    uint32_t cnt_d = 0;
-    if (tid < 256) {
-#pragma unroll
-      for (int w = 0; w < RS_WARPS; w++) { const uint32_t t = whist[w * 256 + tid]; whist[w * 256 + tid] = cnt_d; cnt_d += t; }
-      uint32_t real_d = cnt_d;
-      if (tid == 255) real_d -= (RS_TILE - count);
-      s_gbase[tid] = digit_base[tid] + publish_and_look_back(tile_state, tile, tid, real_d);
-      uint32_t inc = cnt_d;
-#pragma unroll
-      for (int dlt = 1; dlt < 32; dlt <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, inc, dlt); if (lane >= dlt) inc += t; }
-      if (lane == 31) s_scan[warp] = inc;
-      s_dexcl[tid] = inc - cnt_d;
-    }
-    __syncthreads();
-    if (warp == 0) {
-      const uint32_t w = lane < 8 ? s_scan[lane] : 0;
-      uint32_t winc = w;
-#pragma unroll
-      for (int dlt = 1; dlt < 8; dlt <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, winc, dlt); if (lane >= dlt) winc += t; }
-      if (lane < 8) s_scan[lane] = winc - w;
-    }
-    __syncthreads();
-    if (tid < 256) s_dexcl[tid] += s_scan[warp];
-    __syncthreads();
-
-    // 3. scatter into digit order
-#pragma unroll
-    for (int i = 0; i < RS_IPT; i++) {
-      const uint32_t idx = wbase + i * 32 + lane;
-      if (idx < count) {
-        const uint32_t d = dr[i] >> 16;
-        const uint32_t pos = s_dexcl[d] + myhist[d] + (dr[i] & 0xffffu);
-        *reinterpret_cast<ulonglong2 *>(stage + pos) = *reinterpret_cast<const ulonglong2 *>(arr + idx);
-      }
-    }
-    __syncthreads();
-
-    // 4. write out: position j of the staged tile belongs to digit d at global gbase[d] + (j - dexcl[d])
-    for (uint32_t j = tid; j < count; j += RS_THREADS) {
-      const ulonglong2 r = *reinterpret_cast<const ulonglong2 *>(stage + j);
-      const uint32_t d = (uint32_t)((word ? r.y : r.x) >> shift) & mask;
-      *reinterpret_cast<ulonglong2 *>(out + s_gbase[d] + (j - s_dexcl[d])) = r;
-    }
-  }
-}
-
-template <int T, int I, int C>
-static void launch_sweep_tma(kslam_ctx *c, const Rec16 *in, Rec16 *out, uint64_t n, uint32_t shift, uint32_t mask,
-                             uint32_t word, const unsigned long long *base, unsigned long long *state, uint32_t *ticket) {
-  constexpr size_t smem = (size_t)3 * T * I * sizeof(Rec16) + (T / 32) * 256 * sizeof(uint32_t);
-  const uint64_t tiles = (n + (uint64_t)T * I - 1) / ((uint64_t)T * I);
-  static bool attr_set[64] = {false};   // per instantiation
-  if (!(c->device < 64 && attr_set[c->device])) {
-    CUDA_TRY(cudaFuncSetAttribute(k_rs_sweep_tma<T, I, C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    if (c->device < 64) attr_set[c->device] = true;
-  }
-  uint64_t grid = (uint64_t)c->num_sms * C;
-  if (grid > tiles) grid = tiles;
-  k_rs_sweep_tma<T, I, C><<<(unsigned)grid, T, smem, c->stream>>>(in, out, n, shift, mask, word, base, state, ticket, (uint32_t)tiles);
-}
-
 template <int T, int I, int WORD, typename REC = Rec16>
 static void launch_pass2(kslam_ctx *c, const REC *in, REC *out, uint64_t n, uint32_t shift, uint32_t mask,
                          const unsigned long long *base, uint32_t *state, uint32_t *ticket) {
-  // KSLAM_RS_LB=1: the two-level look-back (radix_pass2.cuh). Measured 4 % SLOWER than the flat walk on 32 M / 128 M random
-  // records (2.63 vs 2.53 ms, 9.96 vs 9.57 ms for 8 passes, gpurun_out/r2v_sort.log): the walk is not what bounds a tile.
-  static int flat = -1;
-  if (flat < 0) { const char *e = getenv("KSLAM_RS_LB"); flat = e && atoi(e) == 1 ? 0 : 1; }
   constexpr size_t smem = (size_t)T * I * sizeof(REC) + (T / 32) * 256 * sizeof(uint32_t);
   const uint64_t tiles = (n + (uint64_t)T * I - 1) / ((uint64_t)T * I);
   static bool attr_set[64] = {false};   // per instantiation
@@ -402,21 +251,20 @@ static void launch_pass2(kslam_ctx *c, const REC *in, REC *out, uint64_t n, uint
     CUDA_TRY(cudaFuncSetAttribute(k_rs_pass2<T, I, WORD, REC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (c->device < 64) attr_set[c->device] = true;
   }
-  // the group states sit behind the tile states (the caller's memset covers both)
-  k_rs_pass2<T, I, WORD, REC><<<(unsigned)tiles, T, smem, c->stream>>>(in, out, n, shift, mask, base, state, flat ? nullptr : state + tiles * 256, ticket);
+  k_rs_pass2<T, I, WORD, REC><<<(unsigned)tiles, T, smem, c->stream>>>(in, out, n, shift, mask, base, state, ticket);
 }
 
-template <int T, int I, bool B>
+template <int T, int I>
 static void launch_onesweep(kslam_ctx *c, const Rec16 *in, Rec16 *out, uint64_t n, uint32_t shift, uint32_t mask,
                             uint32_t word, const unsigned long long *base, unsigned long long *state, uint32_t *ticket) {
   constexpr size_t smem = (size_t)T * I * sizeof(Rec16) + (T / 32) * 256 * sizeof(uint32_t);
   const uint64_t tiles = (n + (uint64_t)T * I - 1) / ((uint64_t)T * I);
   static bool attr_set[64] = {false};   // per instantiation
   if (!(c->device < 64 && attr_set[c->device])) {
-    CUDA_TRY(cudaFuncSetAttribute(k_rs_onesweep<T, I, B>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CUDA_TRY(cudaFuncSetAttribute(k_rs_onesweep<T, I>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (c->device < 64) attr_set[c->device] = true;
   }
-  k_rs_onesweep<T, I, B><<<(unsigned)tiles, T, smem, c->stream>>>(in, out, n, shift, mask, word, base, state, ticket);
+  k_rs_onesweep<T, I><<<(unsigned)tiles, T, smem, c->stream>>>(in, out, n, shift, mask, word, base, state, ticket);
 }
 
 Rec16 *radix_sort(kslam_ctx *c, Rec16 *a, Rec16 *b, uint64_t n, uint32_t word, uint32_t lo_bit, uint32_t hi_bit,
@@ -426,22 +274,19 @@ Rec16 *radix_sort(kslam_ctx *c, Rec16 *a, Rec16 *b, uint64_t n, uint32_t word, u
   cudaStream_t st = c->stream;
   // a wide key range is sorted in groups of <= 8 passes
   Rec16 *cur = a, *alt = b;
-  static int cfg = -1;
-  if (cfg < 0) { const char *e = getenv("KSLAM_RS_CFG"); cfg = e ? atoi(e) : 0; }
   PassPlan plan;
   plan.n_passes = 0;
   for (uint32_t s = lo_bit; s < hi_bit && plan.n_passes < RS_MAX_PASSES; s += 8) {
     uint32_t bits = hi_bit - s < 8 ? hi_bit - s : 8;
     plan.shift[plan.n_passes] = s; plan.mask[plan.n_passes] = (1u << bits) - 1; plan.n_passes++;
   }
-  const uint64_t tile_recs = cfg == 2 ? 8192 : ((cfg == 5 || cfg == 7) ? 2048 : 4096);
+  const uint64_t tile_recs = 4096;
   const uint64_t tiles = (n + tile_recs - 1) / tile_recs;
   // layout of sort_hist: [8*256 u64 hist][8 u32 trivial][8 u32 tickets][pad][tiles*256 u64 state / inclusive prefixes]
   // (k_rs_pass2: tiles*256 u32)
   const size_t hist_bytes = RS_MAX_PASSES * 256 * 8, misc_bytes = 128;
-  const bool pass2 = (cfg == 0 || cfg == 10) && n < (1ull << 30);          // its 32-bit tile states hold prefixes below 2^30
-  const int variant = cfg == 10 ? 0 : 1;                   // 1: 256 threads x 16 records (default), 0: 512 x 8 (KSLAM_RS_CFG=10)
-  const size_t state_bytes = tiles * 256 * (pass2 ? 4 : 8) + (pass2 ? (tiles / 16 + 1) * 256 * 4 : 0);   // + k_rs_pass2's group states
+  const bool pass2 = n < (1ull << 30);                     // its 32-bit tile states hold prefixes below 2^30
+  const size_t state_bytes = tiles * 256 * (pass2 ? 4 : 8);
   c->sort_hist.reserve(hist_bytes + misc_bytes + state_bytes);
   unsigned long long *ghist = c->sort_hist.as<unsigned long long>();
   uint32_t *trivial = reinterpret_cast<uint32_t *>((char *)c->sort_hist.p + hist_bytes);
@@ -463,27 +308,9 @@ Rec16 *radix_sort(kslam_ctx *c, Rec16 *a, Rec16 *b, uint64_t n, uint32_t word, u
   for (uint32_t p = 0; p < plan.n_passes; p++) {
     if (h_trivial[p]) continue;   // every record has the same digit: the pass would be the identity
     CUDA_TRY(cudaMemsetAsync(state, 0, state_bytes, st));
-#define RS_LAUNCH(T, I, B) launch_onesweep<T, I, B>(c, cur, alt, n, plan.shift[p], plan.mask[p], word, ghist + p * 256, state, tickets + p)
-    // KSLAM_RS_CFG picks an instance for experiments. Round 2, 32 M / 128 M random records, 8 passes (gpurun_out/r2h_sort_cfgs.log):
-    //   0 k_rs_pass2 256x16 (default) 2.52 / 9.50 ms | 10 k_rs_pass2 512x8 2.70 / 10.1 | 9 k_rs_onesweep 256x16 3.05 / 11.6 |
-    //   6 persistent CTAs + double-buffered bulk copies, 512x8, one CTA per SM 4.08 / 16.4 | 7 the same 256x8, two per SM 6.1 / 24.7
-    // Round 1, 32 M records:
-    //   9 ballots 256x16 3.05 ms (the round-1 default) | 4 MATCH.ANY 256x16 3.46 | 1 ballots 512x8 3.16 | 5 ballots 256x8 (4 CTAs/SM) 3.55 |
-    //   2 MATCH.ANY 512x16 (one CTA/SM). 256x12 at 3 CTAs/SM (3.25) and look-back before the ranking (3.04) were tried and dropped.
-    if (cfg == 6) launch_sweep_tma<512, 8, 1>(c, cur, alt, n, plan.shift[p], plan.mask[p], word, ghist + p * 256, state, tickets + p);
-    else if (cfg == 7) launch_sweep_tma<256, 8, 2>(c, cur, alt, n, plan.shift[p], plan.mask[p], word, ghist + p * 256, state, tickets + p);
-    else if (cfg == 1) RS_LAUNCH(512, 8, true);
-    else if (cfg == 2) RS_LAUNCH(512, 16, false);
-    else if (cfg == 4) RS_LAUNCH(256, 16, false);
-    else if (cfg == 5) RS_LAUNCH(256, 8, true);
-    else if (!pass2) RS_LAUNCH(256, 16, true);
-    else {
-#define RS2_LAUNCH(T, I) (word ? launch_pass2<T, I, 1>(c, cur, alt, n, plan.shift[p], plan.mask[p], ghist + p * 256, reinterpret_cast<uint32_t *>(state), tickets + p) \
-                               : launch_pass2<T, I, 0>(c, cur, alt, n, plan.shift[p], plan.mask[p], ghist + p * 256, reinterpret_cast<uint32_t *>(state), tickets + p))
-      if (variant == 1) RS2_LAUNCH(256, 16); else RS2_LAUNCH(512, 8);
-#undef RS2_LAUNCH
-    }
-#undef RS_LAUNCH
+    if (!pass2) launch_onesweep<256, 16>(c, cur, alt, n, plan.shift[p], plan.mask[p], word, ghist + p * 256, state, tickets + p);
+    else if (word) launch_pass2<256, 16, 1>(c, cur, alt, n, plan.shift[p], plan.mask[p], ghist + p * 256, reinterpret_cast<uint32_t *>(state), tickets + p);
+    else launch_pass2<256, 16, 0>(c, cur, alt, n, plan.shift[p], plan.mask[p], ghist + p * 256, reinterpret_cast<uint32_t *>(state), tickets + p);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
     Rec16 *t = cur; cur = alt; alt = t;
@@ -493,26 +320,24 @@ Rec16 *radix_sort(kslam_ctx *c, Rec16 *a, Rec16 *b, uint64_t n, uint32_t word, u
 }
 
 
-// Bare 8-byte keys (n < 2^30), bits [lo_bit, hi_bit): the same histogram + k_rs_pass2 passes at 16 B per key and pass.
-// KSLAM_RS_U64_IPT=16 picks 4096-key tiles (default 8192).
+// Bare 8-byte keys (n < 2^30), bits [lo_bit, hi_bit): the same histogram + k_rs_pass2 passes at 16 B per key and pass,
+// 8192-key tiles.
 uint64_t *radix_sort_u64(kslam_ctx *c, uint64_t *a, uint64_t *b, uint64_t n, uint32_t lo_bit, uint32_t hi_bit, uint64_t *passes_done) {
   if (n < 2 || hi_bit <= lo_bit) return a;
   if (hi_bit > 64) hi_bit = 64;
   if (n >= (1ull << 30)) throw ArgError{"radix_sort_u64: more than 2^30 keys"};
   cudaStream_t st = c->stream;
   uint64_t *cur = a, *alt = b;
-  static int ipt = -1;
-  if (ipt < 0) { const char *e = getenv("KSLAM_RS_U64_IPT"); ipt = e && atoi(e) == 16 ? 16 : 32; }
   PassPlan plan;
   plan.n_passes = 0;
   for (uint32_t s = lo_bit; s < hi_bit && plan.n_passes < RS_MAX_PASSES; s += 8) {
     uint32_t bits = hi_bit - s < 8 ? hi_bit - s : 8;
     plan.shift[plan.n_passes] = s; plan.mask[plan.n_passes] = (1u << bits) - 1; plan.n_passes++;
   }
-  const uint64_t tile_recs = 256 * (uint64_t)ipt;
+  const uint64_t tile_recs = 8192;
   const uint64_t tiles = (n + tile_recs - 1) / tile_recs;
   const size_t hist_bytes = RS_MAX_PASSES * 256 * 8, misc_bytes = 128;
-  const size_t state_bytes = tiles * 256 * 4 + (tiles / 16 + 1) * 256 * 4;   // tile states + group states
+  const size_t state_bytes = tiles * 256 * 4;
   c->sort_hist.reserve(hist_bytes + misc_bytes + state_bytes);
   unsigned long long *ghist = c->sort_hist.as<unsigned long long>();
   uint32_t *trivial = reinterpret_cast<uint32_t *>((char *)c->sort_hist.p + hist_bytes);
@@ -534,8 +359,7 @@ uint64_t *radix_sort_u64(kslam_ctx *c, uint64_t *a, uint64_t *b, uint64_t n, uin
   for (uint32_t p = 0; p < plan.n_passes; p++) {
     if (h_trivial[p]) continue;
     CUDA_TRY(cudaMemsetAsync(state, 0, state_bytes, st));
-    if (ipt == 16) launch_pass2<256, 16, 0, uint64_t>(c, cur, alt, n, plan.shift[p], plan.mask[p], ghist + p * 256, state, tickets + p);
-    else launch_pass2<256, 32, 0, uint64_t>(c, cur, alt, n, plan.shift[p], plan.mask[p], ghist + p * 256, state, tickets + p);
+    launch_pass2<256, 32, 0, uint64_t>(c, cur, alt, n, plan.shift[p], plan.mask[p], ghist + p * 256, state, tickets + p);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
     uint64_t *t = cur; cur = alt; alt = t;

@@ -676,27 +676,25 @@ int kslam_sam_header(const kslam_sam_db *db, const char *command_line, char **te
 // thread, then into the buffer handed to the caller; taken fresh from malloc every batch, each of those pages is faulted in
 // (and zeroed) again, which costs more than writing the text. The pool keeps the per-thread strings (emptied, capacity
 // kept) and the one largest buffer given back through kslam_sam_free; a second writer running at the same time simply
-// allocates. KSLAM_SAM_NO_POOL=1 switches it off (nothing is retained between batches).
+// allocates.
 struct TextPool {
   std::mutex m;
   std::vector<std::string> parts;
   char *buf = nullptr; size_t cap = 0;
-  const bool off = getenv("KSLAM_SAM_NO_POOL") != nullptr;
   ~TextPool() { free(buf); }
   std::vector<std::string> take_parts(uint32_t threads) {
     std::vector<std::string> p;
-    if (!off) { std::lock_guard<std::mutex> l(m); p.swap(parts); }
+    { std::lock_guard<std::mutex> l(m); p.swap(parts); }
     p.resize(threads);                                       // (a different thread count keeps what fits)
     return p;
   }
   void give_parts(std::vector<std::string> &p) {
-    if (off) return;
     for (std::string &x : p) x.clear();
     std::lock_guard<std::mutex> l(m);
     if (parts.empty()) parts.swap(p);
   }
   char *take_buf(size_t bytes) {
-    if (!off) {
+    {
       std::lock_guard<std::mutex> l(m);
       if (buf && cap >= bytes) { char *b = buf; buf = nullptr; cap = 0; return b; }
     }
@@ -704,7 +702,7 @@ struct TextPool {
   }
   void give_buf(char *b) {
     if (!b) return;
-    const size_t have = off ? 0 : malloc_usable_size(b);
+    const size_t have = malloc_usable_size(b);
     if (have >= (1u << 20)) {                                // small texts (headers) are not worth keeping
       std::lock_guard<std::mutex> l(m);
       if (have > cap) { std::swap(b, buf); cap = have; }

@@ -27,7 +27,6 @@
 //    of the CIGAR pool.
 // Roofline: integer (ALU) pipe; cells/s reported as GCUPS next to the counted ops/cell.
 #include "common.cuh"
-#include <stdlib.h>
 
 #define SW_R 20
 #define SW_MAXCOLS 640
@@ -93,9 +92,6 @@ struct SwScore {
   int32_t match, mismatch, gap_open, gap_extend;   // positive magnitudes, as given
   uint32_t score_threshold; uint32_t report_cigar; uint32_t cigar_cap;
   uint32_t literal;   // 1: scoring parameters outside the plain-Gotoh domain -> every alignment runs k_sw_striped
-  uint32_t max_band;  // widest band tier in use (128; KSLAM_SW_MAX_BAND=64 leaves the tiers of 72-128 diagonals out: ablation)
-  uint32_t anchored;  // 1: reverse sweeps run in the anchored band (KSLAM_SW_REV_ANCHOR=0: the interval [-(rows - a), cols - a])
-  uint32_t ncol;      // 1: windows with code-4 columns run the masked band tiers (KSLAM_SW_NCOL=0: the full-matrix kernel, as before)
 };
 
 struct SwWorkspace {
@@ -141,10 +137,10 @@ __device__ __forceinline__ uint32_t mad_add(uint32_t a, uint32_t one, uint32_t c
   return d;
 }
 
-// smallest tier whose band holds an interval of `width` diagonals; SWT_TIER_NONE when nothing allowed does.
-// level: 1 = 32 only, 2 = 32 and 64, 3 = every width.
-__host__ __device__ __forceinline__ uint32_t tier_of_interval(int32_t width, uint32_t level, const SwScore &sc) {
-  if (width > (int32_t)sc.max_band) return SWT_TIER_NONE;
+// smallest tier whose band holds an interval of `width` diagonals; SWT_TIER_NONE when nothing allowed does (the widest
+// tier is 128 diagonals). level: 1 = 32 only, 2 = 32 and 64, 3 = every width.
+__host__ __device__ __forceinline__ uint32_t tier_of_interval(int32_t width, uint32_t level) {
+  if (width > 128) return SWT_TIER_NONE;
   if (level >= 3) return tier_of_band_width((uint32_t)(width > 0 ? width : 1));
   if (width <= 32) return 3u;
   return (level >= 2 && width <= 64) ? 7u : SWT_TIER_NONE;
@@ -803,7 +799,7 @@ __device__ int32_t diag_lower_bound(const SwPlanes &pl, const SwTask &t, int32_t
 // nothing. level: 1 = 32 only, 2 = 32 and 64, 3 = all five widths.
 __device__ __forceinline__ uint32_t tier_of_width(int32_t rows, int32_t cols, int32_t score, const SwScore &sc, uint32_t level) {
   if (score <= 0) return SWT_TIER_NONE;
-  return tier_of_interval(rows + cols - 2 * ceil_div_pos(score, sc.match) + 1, level, sc);
+  return tier_of_interval(rows + cols - 2 * ceil_div_pos(score, sc.match) + 1, level);
 }
 // One counter per tier, one GLOBAL atomic per (CTA, tier): every thread of the CTA calls this once at the end of its kernel
 // (dead threads with SWT_TIER_NONE). Per-warp global atomics — 5 M warps x up to 6 tiers on six addresses — serialised in
@@ -922,7 +918,7 @@ prepare_seed(uint32_t i, const kslam_seed *__restrict__ seeds, const uint64_t *_
   const uint32_t cls = classify(t.m, t.n, sc);
   t.flags = (s.rev_comp ? SWT_REV : 0u) | (cls << 8);
   if (cls != SWC_NONE && ((g_has_n && !__ldg(&g_has_n[s.entry])) || window_clean(g_nmask, t.w_word, t.w_start, t.n))) t.flags |= SWT_CLEAN;   // (a genome without any code-4 base: no scan)
-  if (use_band && cls == SWC_FAST8 && band_shape_ok(t.m, t.n) && ((t.flags & SWT_CLEAN) || (use_band >= 3 && sc.ncol))) t.flags |= SWT_BAND;
+  if (use_band && cls == SWC_FAST8 && band_shape_ok(t.m, t.n) && ((t.flags & SWT_CLEAN) || use_band >= 3)) t.flags |= SWT_BAND;
   tasks[i] = t;
   // matrix diagonal of the seed's exact 32-mer match: forward seeds put read base i on genome base rel + i; reverse-
   // complement seeds put rc(read) base i there and Align sees the window reversed (SmithWaterman.h:205-208)
@@ -958,7 +954,7 @@ k_sw_prepare_pairs(uint32_t n, const uint64_t *__restrict__ q_offs, const uint64
     const uint32_t cls = classify(t.m, t.n, sc);
     t.flags = cls << 8;
     if (cls != SWC_NONE && window_clean(r_nmask, t.w_word, 0, t.n)) t.flags |= SWT_CLEAN;
-    if (use_band && cls == SWC_FAST8 && band_shape_ok(t.m, t.n) && ((t.flags & SWT_CLEAN) || (use_band >= 3 && sc.ncol))) t.flags |= SWT_BAND;
+    if (use_band && cls == SWC_FAST8 && band_shape_ok(t.m, t.n) && ((t.flags & SWT_CLEAN) || use_band >= 3)) t.flags |= SWT_BAND;
     tasks[i] = t;
     tier = enlist(pl, t, i, cls, 0, false, use_band, sc, res, tier_f, full_keys, slow_list, counts);   // no seed: try the main diagonal
   }
@@ -989,9 +985,9 @@ k_sw_rev_lists(const SwTask *__restrict__ tasks, SwRes *__restrict__ res, uint32
       if (t.flags & SWT_BAND) {
         int32_t lo, hi;
         reverse_band(rows, cols, r.score, sc, &lo, &hi);
-        tier = tier_of_interval(hi - lo + 1, level, sc);
+        tier = tier_of_interval(hi - lo + 1, level);
         if (!(t.flags & SWT_CLEAN)) { if (tier != SWT_TIER_NONE) tier = ncol_tier(tier) | SWT_NCOL; }
-        else if (lo == 0 && hi == 0 && sc.anchored && level >= 3) tier = SWT_TIER_SWEEP;     // (the reverse pass has no trial sweep: this list is k_sw_rev_diagonal's)
+        else if (lo == 0 && hi == 0 && level >= 3) tier = SWT_TIER_SWEEP;     // (the reverse pass has no trial sweep: this list is k_sw_rev_diagonal's)
       }
       if (tier == SWT_TIER_NONE) { const uint32_t k = list_slot(&counts[CNT_FULL]); full_keys[k].key = (uint64_t)cols | ((uint64_t)cls << 16); full_keys[k].val = i; }
     }
@@ -1122,11 +1118,6 @@ static SwScore make_score(const kslam_ctx *c) {
   s.match = (int8_t)c->prm.match; s.mismatch = -(int32_t)(int8_t)(-(int32_t)c->prm.mismatch);
   s.gap_open = c->prm.gap_open; s.gap_extend = c->prm.gap_extend;
   s.literal = kslam_params_fast(&c->prm) ? 0u : 1u;
-  static const char *mb = getenv("KSLAM_SW_MAX_BAND"), *ra = getenv("KSLAM_SW_REV_ANCHOR");
-  s.max_band = mb && atoi(mb) == 64 ? 64u : 128u;
-  s.anchored = ra && atoi(ra) == 0 ? 0u : 1u;
-  static const char *nc = getenv("KSLAM_SW_NCOL");
-  s.ncol = nc && atoi(nc) == 0 ? 0u : 1u;
   s.score_threshold = c->prm.score_threshold; s.report_cigar = c->prm.report_cigar; s.cigar_cap = c->prm.max_cigar_ops;
   return s;
 }
@@ -1506,7 +1497,7 @@ void sw_align_pairs(kslam_ctx *c, uint64_t n64, kslam_overlap *out_dev, uint32_t
 extern "C" int kslam_reverse_band(int32_t rows, int32_t cols, int32_t score, const kslam_params *p, int32_t *lo, int32_t *hi) {
   if (!p || !lo || !hi || rows < 1 || cols < 1 || score < 1 || !kslam_params_fast(p)) return KSLAM_ERR_ARG;
   SwScore sc{};
-  sc.match = (int8_t)p->match; sc.mismatch = p->mismatch; sc.gap_open = p->gap_open; sc.gap_extend = p->gap_extend; sc.anchored = 1;
+  sc.match = (int8_t)p->match; sc.mismatch = p->mismatch; sc.gap_open = p->gap_open; sc.gap_extend = p->gap_extend;
   reverse_band(rows, cols, score, sc, lo, hi);
   return KSLAM_OK;
 }

@@ -110,7 +110,6 @@ __host__ __device__ __forceinline__ int32_t anchored_reach(int32_t other, int32_
 }
 // offsets [lo, hi] of the reverse band of an alignment scoring S whose reversed prefixes are rows x cols
 __host__ __device__ __forceinline__ void reverse_band(int32_t rows, int32_t cols, int32_t S, const SwScore &sc, int32_t *lo, int32_t *hi) {
-  if (!sc.anchored) { const int32_t a = (S + sc.match - 1) / sc.match; *lo = -(rows - a); *hi = cols - a; return; }
   *hi = anchored_reach(rows, cols, S, sc.match, sc.gap_open, sc.gap_extend);
   *lo = -anchored_reach(cols, rows, S, sc.match, sc.gap_open, sc.gap_extend);
 }
@@ -450,9 +449,9 @@ k_sw_band(const SwTask *__restrict__ tasks, const uint32_t *__restrict__ list, u
         o.flags = SWR_FWD_TIER(SWR_TIER_OF_W(W)); o.pad0 = o.pad1 = 0; o.ref_begin = -1; o.read_begin = 0;
         o.score = S; o.ref_end = bcol; o.read_end = brow;
         res[idx] = o;
-      } else if (MODE == 0 && next_list && S > 0 && tier_of_interval(need, level, sc) != SWT_TIER_NONE) {
+      } else if (MODE == 0 && next_list && S > 0 && tier_of_interval(need, level) != SWT_TIER_NONE) {
         res[idx].score = S;         // lower bound: every alignment scoring >= S lies in [-(m - a), n - a]
-        const uint32_t t2 = NCOL ? ncol_tier(tier_of_interval(need, level, sc)) : tier_of_interval(need, level, sc);
+        const uint32_t t2 = NCOL ? ncol_tier(tier_of_interval(need, level)) : tier_of_interval(need, level);
         tier_f[idx] = (uint8_t)(t2 | SWT_SWEPT | (NCOL ? SWT_NCOL : 0u));
         list_slot_keyed(tier2_count, t2 + (NCOL ? SWT_N_DIRECT : 0u));
         next_list[list_slot(next_count)] = idx;

@@ -1,7 +1,6 @@
-"""Worker for tests/test_gpu_parity.py::test_switches_give_the_same_results: the library reads its ablation / fall-back
-switches (KSLAM_SEEDS_EXPAND_AT, KSLAM_SEEDS_16B, KSLAM_SW_NCOL, KSLAM_SW_REV_ANCHOR, KSLAM_SW_MAX_BAND) once per process,
-so every setting runs in a process of its own: whole pipeline on adversarial + related-genome data and the SW stage on
-diverged pairs with code-4 windows, each against the oracle."""
+"""Worker for tests/test_gpu_parity.py::test_switches_give_the_same_results: the library reads its fall-back switches
+(KSLAM_SEEDS_EXPAND_AT, KSLAM_SEEDS_16B) once per process, so every setting runs in a process of its own: whole pipeline
+on adversarial + related-genome data and the SW stage on diverged pairs with code-4 windows, each against the oracle."""
 import os
 import sys
 

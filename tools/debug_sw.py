@@ -1,4 +1,4 @@
-"""GPU debugging aid: the SW stage against the oracle under the ablation switches KSLAM_SW_MAX_BAND / KSLAM_SW_REV_ANCHOR."""
+"""GPU debugging aid: the SW stage against the oracle on diverged pairs, with per-tier counts and the first mismatches."""
 import os, sys, numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tests")); sys.path.insert(0, ROOT)
@@ -8,7 +8,6 @@ pkg = T.load_pkg()
 spec = importlib.util.spec_from_file_location("tgp", os.path.join(ROOT, "tests", "test_gpu_parity.py"))
 tgp = importlib.util.module_from_spec(spec); spec.loader.exec_module(tgp)
 F = ("ref_begin", "ref_end", "query_begin", "query_end", "sw_score")
-print("env", os.environ.get("KSLAM_SW_MAX_BAND"), os.environ.get("KSLAM_SW_REV_ANCHOR"))
 for shape in [(150, 150), (120, 160), (160, 100)]:
     q, qo, r, ro = tgp.diverged_pairs(pkg, 8000, shape[0], shape[1], seed=3)
     want, _ = T.ko_ssw_batch(q, qo, r, ro, T.default_params(report_cigar=0))
