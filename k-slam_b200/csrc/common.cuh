@@ -172,7 +172,7 @@ void exclusive_scan_u32(kslam_ctx *c, const uint32_t *in, uint32_t *out, uint64_
 // join.cu
 void join_and_unique(kslam_ctx *c);
 void seed_sort_unique(kslam_ctx *c);
-uint64_t run_join(kslam_ctx *c, const Rec16 *R, uint64_t n_r, bool match, DevBuf &outbuf, bool compact = false);
+uint64_t run_join(kslam_ctx *c, const Rec16 *R, uint64_t n_r, bool match, DevBuf &outbuf);
 void matches_to_seeds(kslam_ctx *c, const Rec16 *m, uint64_t n, uint32_t id_base);
 // api.cu: sort an extracted genome k-mer list into the reference's order and split it into g_keys / g_vals
 void finish_genome_index(kslam_ctx *c, DevBuf &a, DevBuf &b, uint64_t n);

@@ -43,8 +43,7 @@ static SeedBits seed_bits(const kslam_ctx *c) {
   if (b.rel_bits > 33) b.rel_bits = 33;
   b.ebits = ceil_log2_u64(c->genomes.n > 1 ? c->genomes.n : 2);
   b.rbits = ceil_log2_u64(c->reads.n > 1 ? c->reads.n : 2);
-  static const char *off = getenv("KSLAM_SEEDS_16B");
-  b.compact = (b.rel_bits + b.ebits + b.rbits <= 64 && !(off && atoi(off))) ? 1u : 0u;
+  b.compact = b.rel_bits + b.ebits + b.rbits <= 64 ? 1u : 0u;
   return b;
 }
 __device__ __forceinline__ uint64_t pack_seed64(uint32_t read, uint32_t entry, int32_t rel, uint32_t rc, uint32_t bias, uint32_t rel_bits, uint32_t ebits) {
@@ -88,11 +87,11 @@ __device__ __forceinline__ uint64_t warp_bound(const uint64_t *__restrict__ keys
   return lo + __popc(m);
 }
 
-// MATCH = false: emit packed seeds (needs the read lengths, i.e. the reads live on this GPU).
-// MATCH = true (k-mer-range partitioned database, dist.cu): emit the raw match {read record val, genome record val};
-// the GPU that owns the read turns it into a seed (k_matches_to_seeds) because only it knows the read length.
-// COMPACT: emit one-word seeds (see SeedBits) into out64.
-template <bool MATCH, bool COMPACT>
+// MATCH = false: emit one-word seeds (see SeedBits) into out64 (needs the read lengths, i.e. the reads live on this GPU).
+// MATCH = true: emit the raw match {read record val, genome record val}; k_matches_to_seeds turns it into a 16-byte seed
+// on the GPU that owns the read, because only it knows the read length (k-mer-range partitioned database, dist.cu), or on
+// this GPU when a seed does not fit one word.
+template <bool MATCH>
 __global__ void __launch_bounds__(JN_THREADS)
 k_join(const Rec16 *__restrict__ R, uint64_t n_r, const uint64_t *__restrict__ gkeys,
        const uint64_t *__restrict__ gvals, uint64_t n_g, const uint64_t *__restrict__ read_offs,
@@ -170,9 +169,7 @@ k_join(const Rec16 *__restrict__ R, uint64_t n_r, const uint64_t *__restrict__ g
         uint32_t gf = (uint32_t)gv, g_off = (uint32_t)(gv >> 32);
         uint32_t g_rc = (gf >> 30) & 1;
         uint32_t off = g_rc ? rlen - r_off - KSLAM_K : r_off;           // Overlap.h:185-189
-        if (COMPACT) { out64[o] = pack_seed64(rid, gf & 0x3FFFFFFFu, (int32_t)(g_off - off), g_rc != r_rc, bias, rel_bits, ebits); o++; continue; }
-        Rec16 s = pack_seed(rid, gf & 0x3FFFFFFFu, (int32_t)(g_off - off), g_rc != r_rc, bias);
-        *reinterpret_cast<ulonglong2 *>(out + o) = make_ulonglong2(s.key, s.val);
+        out64[o] = pack_seed64(rid, gf & 0x3FFFFFFFu, (int32_t)(g_off - off), g_rc != r_rc, bias, rel_bits, ebits);
         o++;
       }
     }
@@ -195,6 +192,21 @@ k_unique_flags(const Rec16 *__restrict__ s, uint64_t n, uint32_t *__restrict__ k
       if (d < 3) keep[j] = 0; else { keep[j] = 1; last = rel; }
     }
   }
+}
+
+// kept seed i (packed form r) -> seeds[pos[i]], and ov[pos[i]] = the seed with every alignment field zero
+__device__ __forceinline__ void emit_seed(const Rec16 r, uint32_t bias, const uint32_t *__restrict__ pos, uint64_t i,
+                                          kslam_seed *__restrict__ seeds, kslam_overlap *__restrict__ ov) {
+  kslam_seed o;
+  o.read = (uint32_t)(r.key >> 32); o.entry = (uint32_t)r.key;
+  o.rel = (int32_t)((uint32_t)(r.val >> 1) - bias); o.rev_comp = (uint32_t)(r.val & 1);
+  const uint32_t p = pos[i];
+  seeds[p] = o;
+  kslam_overlap v;
+  v.read = o.read; v.entry = o.entry; v.rel = o.rel; v.rev_comp = o.rev_comp;
+  v.ref_begin = v.ref_end = v.query_begin = v.query_end = 0;
+  v.sw_score = 0; v.cigar_off = 0; v.cigar_len = 0; v.flags = 0;
+  ov[p] = v;
 }
 
 // the same over one-word seeds: a run is the seeds sharing the bits above rel_bits
@@ -220,17 +232,7 @@ k_unique_compact64(const uint64_t *__restrict__ s, uint64_t n, const uint32_t *_
                    uint32_t bias, uint32_t rel_bits, uint32_t ebits, kslam_seed *__restrict__ seeds, kslam_overlap *__restrict__ ov) {
   for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
     if (!keep[i]) continue;
-    const Rec16 r = unpack_seed64(s[i], rel_bits, ebits);
-    kslam_seed o;
-    o.read = (uint32_t)(r.key >> 32); o.entry = (uint32_t)r.key;
-    o.rel = (int32_t)((uint32_t)(r.val >> 1) - bias); o.rev_comp = (uint32_t)(r.val & 1);
-    const uint32_t p = pos[i];
-    seeds[p] = o;
-    kslam_overlap v;
-    v.read = o.read; v.entry = o.entry; v.rel = o.rel; v.rev_comp = o.rev_comp;
-    v.ref_begin = v.ref_end = v.query_begin = v.query_end = 0;
-    v.sw_score = 0; v.cigar_off = 0; v.cigar_len = 0; v.flags = 0;
-    ov[p] = v;
+    emit_seed(unpack_seed64(s[i], rel_bits, ebits), bias, pos, i, seeds, ov);
   }
 }
 
@@ -240,17 +242,7 @@ k_unique_compact(const Rec16 *__restrict__ s, uint64_t n, const uint32_t *__rest
                  kslam_overlap *__restrict__ ov) {
   for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
     if (!keep[i]) continue;
-    Rec16 r = s[i];
-    kslam_seed o;
-    o.read = (uint32_t)(r.key >> 32); o.entry = (uint32_t)r.key;
-    o.rel = (int32_t)((uint32_t)(r.val >> 1) - bias); o.rev_comp = (uint32_t)(r.val & 1);
-    uint32_t p = pos[i];
-    seeds[p] = o;
-    kslam_overlap v;
-    v.read = o.read; v.entry = o.entry; v.rel = o.rel; v.rev_comp = o.rev_comp;
-    v.ref_begin = v.ref_end = v.query_begin = v.query_end = 0;
-    v.sw_score = 0; v.cigar_off = 0; v.cigar_len = 0; v.flags = 0;
-    ov[p] = v;
+    emit_seed(s[i], bias, pos, i, seeds, ov);
   }
 }
 
@@ -285,9 +277,8 @@ void matches_to_seeds(kslam_ctx *c, const Rec16 *m, uint64_t n, uint32_t id_base
 }
 
 // merge-join of n_r sorted read records against the resident genome list; returns the number of records emitted
-// into `outbuf` (packed seeds, or raw matches when `match` is set). The buffer is regrown once on overflow.
-// (compact: one-word seeds, see SeedBits; not with `match`)
-uint64_t run_join(kslam_ctx *c, const Rec16 *R, uint64_t n_r, bool match, DevBuf &outbuf, bool compact) {
+// into `outbuf` (one-word seeds, or raw matches when `match` is set). The buffer is regrown once on overflow.
+uint64_t run_join(kslam_ctx *c, const Rec16 *R, uint64_t n_r, bool match, DevBuf &outbuf) {
   cudaStream_t st = c->stream;
   unsigned long long *d_cnt = c->counters.as<unsigned long long>();
   unsigned long long *h_cnt = c->h_counters.as<unsigned long long>();
@@ -296,21 +287,18 @@ uint64_t run_join(kslam_ctx *c, const Rec16 *R, uint64_t n_r, bool match, DevBuf
   const uint64_t low_mask = sb >= 64 ? 0ull : (~0ull >> sb);
   if (!n_r || !c->n_gk) return 0;
   const SeedBits sb64 = seed_bits(c);
-  const size_t rec = compact ? 8 : sizeof(Rec16);
-  uint64_t cap = outbuf.cap > 64 ? (outbuf.cap - 64) / rec : 0;                  // (64 bytes of slack: radix_pass2.cuh's bulk copies)
+  const size_t rec = match ? sizeof(Rec16) : 8;
+  uint64_t cap = outbuf.cap > 64 ? (outbuf.cap - 64) / rec : 0;                  // (64 bytes of slack: the radix sort's bulk copies)
   if (cap < (1u << 20)) { outbuf.reserve((size_t)(n_r / 8 + (1u << 20)) * rec + 64); cap = (outbuf.cap - 64) / rec; }
   const uint64_t tiles = (n_r + JN_TILE - 1) / JN_TILE;
   for (int attempt = 0; attempt < 2; attempt++) {
     CUDA_TRY(cudaMemsetAsync(d_cnt, 0, 8, st));
     if (match)
-      k_join<true, false><<<(unsigned)tiles, JN_THREADS, 0, st>>>(R, n_r, c->g_keys.as<uint64_t>(), c->g_vals.as<uint64_t>(), c->n_gk,
-                                                                  nullptr, outbuf.as<Rec16>(), cap, d_cnt, bias, low_mask, 0, 0);
-    else if (compact)
-      k_join<false, true><<<(unsigned)tiles, JN_THREADS, 0, st>>>(R, n_r, c->g_keys.as<uint64_t>(), c->g_vals.as<uint64_t>(), c->n_gk,
-                                                                  c->reads.offs.as<uint64_t>(), outbuf.as<Rec16>(), cap, d_cnt, bias, low_mask, sb64.rel_bits, sb64.ebits);
+      k_join<true><<<(unsigned)tiles, JN_THREADS, 0, st>>>(R, n_r, c->g_keys.as<uint64_t>(), c->g_vals.as<uint64_t>(), c->n_gk,
+                                                           nullptr, outbuf.as<Rec16>(), cap, d_cnt, bias, low_mask, 0, 0);
     else
-      k_join<false, false><<<(unsigned)tiles, JN_THREADS, 0, st>>>(R, n_r, c->g_keys.as<uint64_t>(), c->g_vals.as<uint64_t>(), c->n_gk,
-                                                                   c->reads.offs.as<uint64_t>(), outbuf.as<Rec16>(), cap, d_cnt, bias, low_mask, 0, 0);
+      k_join<false><<<(unsigned)tiles, JN_THREADS, 0, st>>>(R, n_r, c->g_keys.as<uint64_t>(), c->g_vals.as<uint64_t>(), c->n_gk,
+                                                            c->reads.offs.as<uint64_t>(), outbuf.as<Rec16>(), cap, d_cnt, bias, low_mask, sb64.rel_bits, sb64.ebits);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
     read_small(c, h_cnt, d_cnt, 8);
@@ -329,7 +317,12 @@ void join_and_unique(kslam_ctx *c) {
   c->n_raw = 0; c->n_seeds = 0;
   cudaEvent_t e0 = tm_mark(c);
   c->seeds_compact = seed_bits(c).compact != 0;
-  c->n_raw = run_join(c, c->sorted_rk, c->n_rk, false, c->seedA, c->seeds_compact);
+  if (c->seeds_compact) {
+    c->n_raw = run_join(c, c->sorted_rk, c->n_rk, false, c->seedA);
+  } else {   // 16-byte seeds: raw matches, then the partitioned path's conversion (read ids here are batch-local)
+    const uint64_t n_m = run_join(c, c->sorted_rk, c->n_rk, true, c->seedB);
+    matches_to_seeds(c, c->seedB.as<Rec16>(), n_m, 0);
+  }
   cudaEvent_t e1 = tm_mark(c);
   seed_sort_unique(c);
   c->tm.ms_join = tm_ms(e0, e1);
@@ -348,22 +341,13 @@ void seed_sort_unique(kslam_ctx *c) {
   c->tm.n_raw_seeds = c->n_raw;
   cudaEvent_t e2 = e1, e3 = e1;
   const SeedBits sb = seed_bits(c);
-  uint64_t eblocks = (c->n_raw + 255) / 256;
-  if (eblocks > (uint64_t)c->num_sms * 16) eblocks = (uint64_t)c->num_sms * 16;
-  static const char *xe = getenv("KSLAM_SEEDS_EXPAND_AT");            // (tests: take the fall-back below on small inputs)
-  const uint64_t expand_at = xe && atoll(xe) > 0 ? (uint64_t)atoll(xe) : (1ull << 30);
-  if (c->n_raw && c->seeds_compact && c->n_raw >= expand_at) {        // beyond radix_sort_u64's range: back to 16-byte records
-    c->seedB.reserve((size_t)c->n_raw * sizeof(Rec16));
-    k_seeds_expand<<<(unsigned)eblocks, 256, 0, st>>>(c->seedA.as<uint64_t>(), c->n_raw, sb.rel_bits, sb.ebits, c->seedB.as<Rec16>());
-    c->launches++;
-    DevBuf t = c->seedA; c->seedA = c->seedB; c->seedB = t;
-    c->seeds_compact = false;
-  }
+  uint64_t blocks = (c->n_raw + 255) / 256;
+  if (blocks > (uint64_t)c->num_sms * 16) blocks = (uint64_t)c->num_sms * 16;
   if (c->n_raw && c->seeds_compact) {
     c->seedB.reserve((size_t)c->n_raw * 8 + 64);
     if (c->keep_taps) {   // tap: raw seeds before sorting (order is not contractual), in the 16-byte form the getter unpacks
       c->raw_seeds.reserve((size_t)c->n_raw * sizeof(Rec16));
-      k_seeds_expand<<<(unsigned)eblocks, 256, 0, st>>>(c->seedA.as<uint64_t>(), c->n_raw, sb.rel_bits, sb.ebits, c->raw_seeds.as<Rec16>());
+      k_seeds_expand<<<(unsigned)blocks, 256, 0, st>>>(c->seedA.as<uint64_t>(), c->n_raw, sb.rel_bits, sb.ebits, c->raw_seeds.as<Rec16>());
       c->launches++;
     }
     uint64_t passes = 0;
@@ -373,7 +357,7 @@ void seed_sort_unique(kslam_ctx *c) {
     c->seed_keep.reserve((size_t)c->n_raw * 8 + 64);
     uint32_t *keep = c->seed_keep.as<uint32_t>();
     uint32_t *pos = keep + c->n_raw;
-    k_unique_flags64<<<(unsigned)eblocks, 256, 0, st>>>(cur, c->n_raw, sb.rel_bits, keep);
+    k_unique_flags64<<<(unsigned)blocks, 256, 0, st>>>(cur, c->n_raw, sb.rel_bits, keep);
     c->launches++;
     exclusive_scan_u32(c, keep, pos, c->n_raw, (uint64_t *)(d_cnt + 1));
     read_small(c, h_cnt + 1, d_cnt + 1, 8);
@@ -381,7 +365,7 @@ void seed_sort_unique(kslam_ctx *c) {
     c->n_seeds = h_cnt[1];
     c->seeds.reserve((size_t)c->n_seeds * sizeof(kslam_seed) + 64);
     c->ov.reserve((size_t)c->n_seeds * sizeof(kslam_overlap) + 64);
-    k_unique_compact64<<<(unsigned)eblocks, 256, 0, st>>>(cur, c->n_raw, keep, pos, bias, sb.rel_bits, sb.ebits, c->seeds.as<kslam_seed>(),
+    k_unique_compact64<<<(unsigned)blocks, 256, 0, st>>>(cur, c->n_raw, keep, pos, bias, sb.rel_bits, sb.ebits, c->seeds.as<kslam_seed>(),
                                                          c->ov.as<kslam_overlap>());
     c->launches++;
     CUDA_TRY(cudaGetLastError());
@@ -394,24 +378,18 @@ void seed_sort_unique(kslam_ctx *c) {
     }
     // LSD over the 128-bit composite (read, entry, rel, rev_comp): low word first, then the high word
     uint64_t passes = 0;
-    uint32_t rel_bits = ceil_log2_u64((uint64_t)c->max_genome_len + 2ull * bias + 2) + 1;
-    if (rel_bits > 33) rel_bits = 33;
     Rec16 *a = c->seedA.as<Rec16>(), *b = c->seedB.as<Rec16>();
-    Rec16 *cur = radix_sort(c, a, b, c->n_raw, 1, 0, rel_bits, &passes);
+    Rec16 *cur = radix_sort(c, a, b, c->n_raw, 1, 0, sb.rel_bits, &passes);
     Rec16 *alt = cur == a ? b : a;
-    uint32_t ebits = ceil_log2_u64(c->genomes.n > 1 ? c->genomes.n : 2);
-    cur = radix_sort(c, cur, alt, c->n_raw, 0, 0, ebits, &passes);
+    cur = radix_sort(c, cur, alt, c->n_raw, 0, 0, sb.ebits, &passes);
     alt = cur == a ? b : a;
-    uint32_t rbits = ceil_log2_u64(c->reads.n > 1 ? c->reads.n : 2);
-    cur = radix_sort(c, cur, alt, c->n_raw, 0, 32, 32 + rbits, &passes);
+    cur = radix_sort(c, cur, alt, c->n_raw, 0, 32, 32 + sb.rbits, &passes);
     c->tm.n_sort_passes += passes;
     e2 = tm_mark(c);
     // unique
     c->seed_keep.reserve((size_t)c->n_raw * 8 + 64);
     uint32_t *keep = c->seed_keep.as<uint32_t>();
     uint32_t *pos = keep + c->n_raw;
-    uint64_t blocks = (c->n_raw + 255) / 256, maxb = (uint64_t)c->num_sms * 16;
-    if (blocks > maxb) blocks = maxb;
     k_unique_flags<<<(unsigned)blocks, 256, 0, st>>>(cur, c->n_raw, keep);
     c->launches++;
     exclusive_scan_u32(c, keep, pos, c->n_raw, (uint64_t *)(d_cnt + 1));

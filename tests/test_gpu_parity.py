@@ -1,6 +1,4 @@
 """GPU tier: the CUDA path (through the C ABI) against the oracle and the committed golden vectors."""
-import os
-
 import numpy as np
 import pytest
 
@@ -453,17 +451,6 @@ def test_ssw_windows_with_code4_columns(pkg, shape, cigar):
     assert tm["n_sw_slow"] == 0
     assert tm["n_sw_band"] == 10_000, tm["n_sw_band"]          # every window is band-eligible, clean or not
     assert tm["n_sw_fast"] < 9_000, tm["n_sw_fast"]            # (what is left: trial sweeps that bound nothing <= 128 diagonals)
-
-
-@pytest.mark.parametrize("env", [{"KSLAM_SEEDS_EXPAND_AT": "1000"}, {"KSLAM_SEEDS_16B": "1"}])
-def test_switches_give_the_same_results(pkg, env):
-    """Both fall-back switches of the library leave the results bit-identical to the oracle: seeds expanded back to
-    16-byte records (the path of batches with >= 2^30 raw seeds) and 16-byte seeds from the start."""
-    import subprocess
-    import sys
-    worker = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_env_worker.py")
-    r = subprocess.run([sys.executable, worker], env=dict(os.environ, **env), capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0 and "SWITCHES-OK" in r.stdout, (r.stdout[-2000:], r.stderr[-4000:])
 
 
 def test_radix_sort_matches_numpy(pkg):
