@@ -6,9 +6,10 @@
 // :594-792), then un-flips coordinates for reverse-complement seeds.
 //
 // Here (DESIGN.md §3.4):
-//  * k_sw_band<MODE, W> (sw_band.cuh): one THREAD owns two alignments packed in the halves of s16x2 registers and sweeps a
-//    band of W = 8 / 16 / 32 / 48 / 64 diagonals that provably contains every optimal alignment (the bound comes from
-//    diag_lower_bound, from a first 32-wide sweep, or — reverse pass — from the forward score). Most alignments.
+//  * k_sw_band<MODE, WP, PARTS> (sw_band.cuh): one THREAD (or 2-4 neighbouring lanes) owns two alignments packed in the
+//    halves of s16x2 registers and sweeps a band of one of twelve tiers of 8-128 diagonals that provably contains every
+//    optimal alignment (the bound comes from diag_lower_bound, from a first 32-wide sweep, or — reverse pass — from the
+//    forward score). Most alignments.
 //  * k_sw_fast<LANES, REVERSE>: a group of LANES threads owns two alignments; each lane keeps SW_R=20 query rows (H, E and a
 //    4-byte score profile per row) in registers and the group sweeps the columns as an anti-diagonal wavefront (lane g works
 //    on column t-g at step t, boundary H/F handed down with shuffles). The full matrix, for what no band can hold.
@@ -19,7 +20,9 @@
 //    step / row counter reproduces SSW's tie rules exactly (first column, then smallest row). REVERSE runs the same sweep
 //    over the reversed prefixes and records the first column reaching the forward score (ssw.c:905-923). No tensor cores:
 //    nothing here is a dense contraction.
-//  * k_sw_slow: exact scalar fallback (one thread per alignment) for shapes outside the packed kernels' range.
+//  * k_sw_striped: SSW's striped byte / word kernels restated lane for lane (16 threads per alignment), for every
+//    alignment the packed kernels cannot take: parameters outside the plain-Gotoh domain or the packed cells' range,
+//    reads or windows over 640 bases, scores the 16-bit cells cannot hold.
 //  * k_sw_traceback: pass 0 emits "len M" when the sub-rectangle's main diagonal already scores the alignment score
 //    (word-parallel XOR + popcount); the rest runs a literal restatement of banded_sw (ssw.c:594-792) — rolling h_b/e_b/h_c
 //    arrays with the reference's index maps (set_u/set_d), direction bytes, band doubling, traceback quirks — one thread
@@ -63,7 +66,7 @@ struct __align__(16) SwRes {
 //   lanes     1   1   1   1   2x20  2x24  2x28  2x32  3x24  4x20  3x32  4x32      (k_sw_band<MODE, slots per lane, lanes>)
 // 12 = 32 diagonals centred, sweep-and-verify; 255 = not in a band list. A forward tier byte with SWT_SWEPT set: the
 // alignment went through the 32-wide trial sweep first and then into that tier with the score the sweep found as its bound.
-// Tier code in SwRes.flags: tier + 1, 0 = full-matrix / scalar kernel.
+// Tier code in SwRes.flags: tier + 1, 0 = full-matrix / striped kernel.
 // A tier byte with SWT_NCOL set: the window has code-4 columns (score 0 against every row, ssw_cpp.cpp:43-48), which a
 // PRMT column selector cannot express; such alignments run the NCOL instances of the kernel (a second PRMT per cell masks
 // the score), which exist for the tiers of 16, 32, 64 and 128 diagonals and the trial sweep, and have lists of their own
@@ -95,7 +98,7 @@ struct SwScore {
 };
 
 struct SwWorkspace {
-  DevBuf tasks, res, keys, keys2, items, lists, bandbytes, tb_scratch, tier;
+  DevBuf tasks, res, keys, keys2, items, lists, tb_scratch, tier;
   uint64_t n = 0;
 };
 
@@ -147,7 +150,6 @@ __host__ __device__ __forceinline__ uint32_t tier_of_interval(int32_t width, uin
 }
 
 // counters (u32) in c->counters + 32
-#define CNT_BAND 0
 #define CNT_FULL 1
 #define CNT_SLOW 2
 #define CNT_RETRY 4
@@ -314,55 +316,6 @@ k_sw_fast(const SwTask *__restrict__ tasks, const uint2 *__restrict__ items, uin
   }
 }
 
-// ---------------------------------------------------------------- slow exact fallback
-// One thread per alignment, plain Gotoh in int32 with SSW's tie rules; H/E rows live in global scratch.
-__device__ void sw_scan_slow(const SwPlanes &pl, const SwTask &t, const SwScore &sc, bool reverse, int32_t rows,
-                             int32_t cols, int32_t ref_end, int32_t read_end, int32_t terminate, int32_t *H,
-                             int32_t *E, uint32_t stride, int32_t *o_score, int32_t *o_ref, int32_t *o_read) {
-  int32_t best = 0, bref = -1, bread = 0;
-  for (int32_t i = 0; i < rows; i++) { H[(size_t)i * stride] = 0; E[(size_t)i * stride] = 0; }
-  for (int32_t c = 0; c < cols; c++) {
-    uint32_t wc = w_code(pl, t, reverse ? (uint32_t)(ref_end - c) : (uint32_t)c);
-    int32_t F = 0, diag = 0, colmax = 0, colrow = 0;
-    for (int32_t i = 0; i < rows; i++) {
-      uint32_t qc = q_code(pl, t, reverse ? (uint32_t)(read_end - i) : (uint32_t)i);
-      int32_t s = (wc == 4 || qc == 4) ? 0 : (wc == qc ? sc.match : -sc.mismatch);
-      int32_t h = diag + s, e = E[(size_t)i * stride];
-      if (h < e) h = e; if (h < F) h = F; if (h < 0) h = 0;
-      diag = H[(size_t)i * stride]; H[(size_t)i * stride] = h;
-      if (h > colmax) { colmax = h; colrow = i; }
-      int32_t hg = h - sc.gap_open; if (hg < 0) hg = 0;
-      e -= sc.gap_extend; if (e < 0) e = 0; E[(size_t)i * stride] = e > hg ? e : hg;
-      F -= sc.gap_extend; if (F < 0) F = 0; if (F < hg) F = hg;
-    }
-    if (colmax > best) { best = colmax; bref = c; bread = colrow; }
-    if (terminate >= 0 && colmax == terminate) break;
-  }
-  *o_score = best; *o_ref = bref; *o_read = bread;
-}
-
-__global__ void __launch_bounds__(128)
-k_sw_slow(const SwTask *__restrict__ tasks, const uint32_t *__restrict__ list, uint32_t n_list, SwPlanes pl,
-          SwScore sc, SwRes *__restrict__ res, int32_t *__restrict__ scratch, uint32_t max_rows) {
-  const uint32_t nthreads = gridDim.x * blockDim.x;
-  const uint32_t tid = blockIdx.x * blockDim.x + threadIdx.x;
-  int32_t *H = scratch + tid, *E = scratch + (size_t)max_rows * nthreads + tid;
-  for (uint32_t k = tid; k < n_list; k += nthreads) {
-    const uint32_t idx = list[k];
-    const SwTask t = tasks[idx];
-    SwRes o; o.flags = 0; o.pad0 = o.pad1 = 0; o.ref_begin = -1; o.read_begin = 0;
-    int32_t s, r, q;
-    sw_scan_slow(pl, t, sc, false, (int32_t)t.m, (int32_t)t.n, 0, 0, -1, H, E, nthreads, &s, &r, &q);
-    o.score = s; o.ref_end = r; o.read_end = q;
-    if (s > 0) {
-      int32_t s2, r2, q2;
-      sw_scan_slow(pl, t, sc, true, q + 1, r + 1, r, q, s, H, E, nthreads, &s2, &r2, &q2);
-      o.ref_begin = r - r2; o.read_begin = q - q2;
-    } else { o.ref_end = -1; o.read_end = 0; }
-    res[idx] = o;
-  }
-}
-
 // ---------------------------------------------------------------- literal striped SSW (any scoring parameters)
 // SSW's striped kernels equal plain Gotoh only when gap_extend < gap_open and mismatch <= 2 * gap_extend (DESIGN.md
 // §3.4). Outside that domain the result depends on details of the striping itself: E is updated from the H value BEFORE
@@ -372,8 +325,10 @@ k_sw_slow(const SwTask *__restrict__ tasks, const uint32_t *__restrict__ list, u
 // restates both kernels lane for lane — a group of 16 threads IS the 16 byte lanes (8 of them the word lanes), vector j
 // of lane l holds query row j + l * segLen (ssw.c:105-133,385-406), _mm_slli_si128 is a shuffle-up inside the group,
 // movemask tests are ballots — and then ssw_align's control flow: byte pass, word pass on overflow (ssw.c:868-877),
-// reverse pass over the reversed prefixes with the forward score as `terminate` (ssw.c:905-923). Speed is secondary
-// here (it only runs for non-default --match-score / --mismatch-penalty / --gap-* combinations); exactness is not.
+// reverse pass over the reversed prefixes with the forward score as `terminate` (ssw.c:905-923). Inside the domain this
+// is plain Gotoh up to the word pass's saturation at 32767, which it keeps as the reference does. Speed is secondary
+// here (it runs only for what the packed kernels cannot take: non-default --match-score / --mismatch-penalty / --gap-*
+// combinations, reads or windows over 640 bases); exactness is not.
 #define STR_GROUPS 8          // 16-lane groups per CTA
 #define STR_SMEM_SEGS 24      // state of reads up to 192 bases (word mode) lives in shared memory, longer ones in global scratch
 
@@ -794,9 +749,9 @@ __device__ int32_t diag_lower_bound(const SwPlanes &pl, const SwTask &t, int32_t
   }
   return best;
 }
-// smallest direct tier (0..4 = 8 / 16 / 32 / 48 / 64 diagonals) whose band holds [-(rows - a), cols - a],
+// smallest direct tier (0..11 = 8-128 diagonals, table at the top of this file) whose band holds [-(rows - a), cols - a],
 // a = ceil(score / match); SWT_TIER_NONE when the interval is wider than the widest tier allowed or the score says
-// nothing. level: 1 = 32 only, 2 = 32 and 64, 3 = all five widths.
+// nothing. level: 1 = 32 only, 2 = 32 and 64, 3 = all twelve widths.
 __device__ __forceinline__ uint32_t tier_of_width(int32_t rows, int32_t cols, int32_t score, const SwScore &sc, uint32_t level) {
   if (score <= 0) return SWT_TIER_NONE;
   return tier_of_interval(rows + cols - 2 * ceil_div_pos(score, sc.match) + 1, level);
@@ -814,9 +769,11 @@ __device__ __forceinline__ void count_tier_block(uint32_t tier, uint32_t *__rest
   if (threadIdx.x < SWT_N_LISTS && s_cnt[threadIdx.x]) atomicAdd(&counts[CNT_TIER + threadIdx.x], s_cnt[threadIdx.x]);
 }
 
+// Kernel class of an alignment. SWC_SLOW (the slow list, run by k_sw_striped): parameters outside the plain-Gotoh domain,
+// and shapes or scores the packed full-matrix kernels cannot hold.
 __device__ __forceinline__ uint32_t classify(uint32_t m, uint32_t n, const SwScore &sc) {
   if (m == 0 || n == 0) return SWC_NONE;
-  if (sc.literal) return SWC_SLOW;     // the slow list is run by k_sw_striped for such parameters
+  if (sc.literal) return SWC_SLOW;
   const uint32_t mn = m < n ? m : n;
   // 16-bit cells: the largest possible score, scaled by 32 and biased (sw_bias), must stay below 2^15
   const bool score_ok = sc.match >= 1 && sc.match * 32 <= 127 && sc.mismatch * 32 <= 128 && sc.gap_open <= 100 && sc.gap_extend <= 100 &&
@@ -853,7 +810,7 @@ __device__ __forceinline__ bool window_clean(const uint32_t *__restrict__ nmask,
 // `tiers` on, the seed-diagonal lower bound L picks the narrowest band that provably holds every optimal alignment
 // (res[].score = L is what MODE 2 of k_sw_band places the band with); otherwise, or when L allows nothing <= 64
 // diagonals (e.g. an indel splits the read over two diagonals), the 32-wide sweep-and-verify tier.
-__device__ __forceinline__ uint32_t enlist(const SwPlanes &pl, const SwTask &t, uint32_t i, uint32_t cls, int32_t d0, bool seeded, uint32_t level,
+__device__ __forceinline__ uint32_t enlist(const SwPlanes &pl, const SwTask &t, uint32_t i, uint32_t cls, int32_t d0, uint32_t level,
                                        const SwScore &sc, SwRes *__restrict__ res, uint8_t *__restrict__ tier_f,
                                        Rec16 *__restrict__ full_keys, uint32_t *__restrict__ slow_list, uint32_t *__restrict__ counts) {
   uint32_t tier = SWT_TIER_NONE;
@@ -923,7 +880,7 @@ prepare_seed(uint32_t i, const kslam_seed *__restrict__ seeds, const uint64_t *_
   // matrix diagonal of the seed's exact 32-mer match: forward seeds put read base i on genome base rel + i; reverse-
   // complement seeds put rc(read) base i there and Align sees the window reversed (SmithWaterman.h:205-208)
   const int32_t d0 = s.rev_comp ? (int32_t)t.w_start + (int32_t)t.n - s.rel - (int32_t)t.m : s.rel - (int32_t)t.w_start;
-  return enlist(pl, t, i, cls, d0, true, use_band, sc, res, tier_f, full_keys, slow_list, counts);
+  return enlist(pl, t, i, cls, d0, use_band, sc, res, tier_f, full_keys, slow_list, counts);
 }
 __global__ void __launch_bounds__(256)
 k_sw_prepare_seeds(const kslam_seed *__restrict__ seeds, uint32_t n, const uint64_t *__restrict__ r_offs,
@@ -956,7 +913,7 @@ k_sw_prepare_pairs(uint32_t n, const uint64_t *__restrict__ q_offs, const uint64
     if (cls != SWC_NONE && window_clean(r_nmask, t.w_word, 0, t.n)) t.flags |= SWT_CLEAN;
     if (use_band && cls == SWC_FAST8 && band_shape_ok(t.m, t.n) && ((t.flags & SWT_CLEAN) || use_band >= 3)) t.flags |= SWT_BAND;
     tasks[i] = t;
-    tier = enlist(pl, t, i, cls, 0, false, use_band, sc, res, tier_f, full_keys, slow_list, counts);   // no seed: try the main diagonal
+    tier = enlist(pl, t, i, cls, 0, use_band, sc, res, tier_f, full_keys, slow_list, counts);   // no seed: try the main diagonal
   }
   count_tier_block(tier, counts);
 }
@@ -1192,9 +1149,10 @@ static void make_tier_lists(kslam_ctx *c, uint32_t n, const uint8_t *tier, const
   for (uint32_t t = 0; t < n_tiers; t++) cnt[t] = h_counts[cnt_at + t];
 }
 
-// one direction (forward or reverse) over the tier lists: the direct tiers (band placed exactly, 8 / 16 / 32 / 64
-// diagonals), forward only: the 32-wide sweep-and-verify tier and the 64-wide tier for what it could not prove but
-// bounded; then every remaining alignment through the full-matrix kernel, bucketed by column count
+// one direction (forward or reverse) over the tier lists: the direct tiers (band placed exactly, 8-128 diagonals) and
+// their NCOL instances; reverse only: the one-diagonal list through k_sw_rev_diagonal, what it cannot settle in the
+// 8-diagonal tier; forward only: the 32-wide trial sweep, and what it bounds but cannot prove through the direct tiers
+// in a second round; then every remaining alignment through the full-matrix kernel, bucketed by column count
 template <bool REVERSE>
 static void sw_pass(kslam_ctx *c, uint32_t n, const SwPlanes &pl, const SwScore &sc, const uint32_t cnt[SWT_N_LISTS], uint32_t *d_counts,
                     uint32_t *h_counts, uint64_t *n_band64_via_sweep, uint64_t *n_full_done) {
@@ -1318,7 +1276,7 @@ static void sw_run(kslam_ctx *c, uint32_t n, const SwPlanes &pl, kslam_overlap *
   cudaEvent_t e2 = tm_mark(c);
 
   // ---- reverse
-  CUDA_TRY(cudaMemsetAsync(d_counts + CNT_BAND, 0, 8, st));   // band + full counters
+  CUDA_TRY(cudaMemsetAsync(d_counts + CNT_FULL, 0, 4, st));
   CUDA_TRY(cudaMemsetAsync(d_counts + CNT_TIER, 0, SWT_N_LISTS * 4, st));
   k_sw_rev_lists<<<nb, 256, 0, st>>>(tasks, res, n, sc, pl, tier_r, sw_level(c), w->keys.as<Rec16>(), d_counts);
   c->launches++;
@@ -1329,21 +1287,15 @@ static void sw_run(kslam_ctx *c, uint32_t n, const SwPlanes &pl, kslam_overlap *
   for (uint32_t t = 0; t < SWT_N_DIRECT; t++) { c->tm.n_sw_rev_tier[t] = cnt[t] + cnt[SWT_N_TIERS + t]; c->tm.n_sw_band_rev += cnt[t] + cnt[SWT_N_TIERS + t]; }
   cudaEvent_t e3 = tm_mark(c);
 
-  // ---- exact scalar fallback for shapes outside the fast kernels
+  // ---- the slow list (classify): k_sw_striped gives SSW's result for every parameter set
   if (n_slow) {
     uint32_t max_rows = c->reads_loaded ? c->reads.max_len : 0;
     if (c->sw_loaded && c->swq.max_len > max_rows) max_rows = c->swq.max_len;
-    uint32_t blocks = (n_slow + 127) / 128; if (blocks > (uint32_t)c->num_sms * 4) blocks = c->num_sms * 4;
-    if (sc.literal) {
-      const uint32_t seg_cap = (max_rows + 7) / 8 + 1;
-      blocks = (n_slow + STR_GROUPS - 1) / STR_GROUPS; if (blocks > (uint32_t)c->num_sms * 8) blocks = c->num_sms * 8;
-      if (seg_cap > STR_SMEM_SEGS) w->tb_scratch.reserve((size_t)blocks * STR_GROUPS * 5 * seg_cap * 16 * 2 + 64);
-      else w->tb_scratch.reserve(64);
-      k_sw_striped<<<blocks, STR_GROUPS * 16, 0, st>>>(tasks, slow_list, n_slow, pl, sc, res, w->tb_scratch.as<int16_t>(), seg_cap);
-    } else {
-    w->tb_scratch.reserve((size_t)blocks * 128 * max_rows * 8 + 64);
-    k_sw_slow<<<blocks, 128, 0, st>>>(tasks, slow_list, n_slow, pl, sc, res, w->tb_scratch.as<int32_t>(), max_rows);
-    }
+    const uint32_t seg_cap = (max_rows + 7) / 8 + 1;
+    uint32_t blocks = (n_slow + STR_GROUPS - 1) / STR_GROUPS; if (blocks > (uint32_t)c->num_sms * 8) blocks = c->num_sms * 8;
+    if (seg_cap > STR_SMEM_SEGS) w->tb_scratch.reserve((size_t)blocks * STR_GROUPS * 5 * seg_cap * 16 * 2 + 64);
+    else w->tb_scratch.reserve(64);
+    k_sw_striped<<<blocks, STR_GROUPS * 16, 0, st>>>(tasks, slow_list, n_slow, pl, sc, res, w->tb_scratch.as<int16_t>(), seg_cap);
     c->launches++;
     CUDA_TRY(cudaGetLastError());
   }
@@ -1505,6 +1457,6 @@ extern "C" int kslam_reverse_band(int32_t rows, int32_t cols, int32_t score, con
 void sw_workspace_free(kslam_ctx *c) {
   if (!c->sw) return;
   c->sw->tasks.release(); c->sw->res.release(); c->sw->keys.release(); c->sw->keys2.release();
-  c->sw->items.release(); c->sw->lists.release(); c->sw->bandbytes.release(); c->sw->tb_scratch.release(); c->sw->tier.release();
+  c->sw->items.release(); c->sw->lists.release(); c->sw->tb_scratch.release(); c->sw->tier.release();
   delete c->sw; c->sw = nullptr;
 }

@@ -133,16 +133,14 @@ __device__ __forceinline__ BandGeo band_geo(const SwTask &t, const SwRes &r, con
 }
 
 // ---- selector streams ------------------------------------------------------------------------------------
-// Column stream of one alignment: byte k = PRMT selector byte of matrix column j = k + c0 in the sweep's orientation —
-// for alignment A (low half of the s16x2 registers) nibbles {w, 8|w}: copy byte w of profile A and replicate its sign;
-// for B nibbles {4|w, 12|w} on profile B; columns outside the matrix replicate the sign of byte 0 (score 0 or -1, never
-// positive). 32 columns are fetched as one oriented 2-bit word and turned into bytes four at a time by one PRMT.
+// Column stream of one alignment: nibble k = 2-bit code of matrix column j = k + c0 in the sweep's orientation, 4 =
+// outside the matrix, eight columns per word; col_selectors() turns four nibbles into PRMT selector bytes for
+// alignment A or B. 32 columns are fetched as one oriented 2-bit word.
 // NCOL: the window may hold code-4 bases; their columns get nibble 5 (the selector LUTs answer it with a byte whose bit 7
 // is clear, which make_selector turns into a masking second selector).
 template <int MODE, bool NCOL>
-__device__ __forceinline__ void fill_col_stream(const SwPlanes &pl, const SwTask &t, const SwRes &r, const BandGeo &g, bool is_b,
+__device__ __forceinline__ void fill_col_stream(const SwPlanes &pl, const SwTask &t, const SwRes &r, const BandGeo &g,
                                                 int32_t kmax, uint32_t *__restrict__ col) {
-  (void)is_b;                                               // (the streams hold codes; col_selectors() makes them selectors)
   constexpr bool REVERSE = MODE == 1;
   const bool rev = (t.flags & SWT_REV) != 0;
   // genome position of matrix column j is P0 + sg * j (window reversal and the reverse sweep both flip the sign)
@@ -287,8 +285,8 @@ k_sw_band(const SwTask *__restrict__ tasks, const uint32_t *__restrict__ list, u
 
   // ---- unpack this thread's selector streams (low half = alignment A, high half = B; an unpaired last slot runs the
   // same alignment in both halves and drops the second result)
-  fill_col_stream<MODE, NCOL>(pl, ta, ra, ga, false, rows4 + WP, colA);
-  fill_col_stream<MODE, NCOL>(pl, tb, rb, gb, true, rows4 + WP, colB);
+  fill_col_stream<MODE, NCOL>(pl, ta, ra, ga, rows4 + WP, colA);
+  fill_col_stream<MODE, NCOL>(pl, tb, rb, gb, rows4 + WP, colB);
   for (int32_t g = 0; 32 * g < rows4 + 4; g++) {
     uint32_t qa[8], qb[8];
     q_group<MODE>(pl, ta, rows[0], g, qa);

@@ -160,7 +160,7 @@ def test_empty_and_ragged_inputs(pkg):
 @pytest.mark.parametrize("read_len,frag,kernel", [(251, 500, "fast"), (301, 560, "fast"), (500, 590, "fast"), (700, 900, "slow")])
 def test_long_reads(pkg, read_len, frag, kernel):
     """Reads beyond the 160 rows of the 8-lane full-matrix kernel: 161-320 bases run the 16-lane instance (250 / 300-bp
-    MiSeq reads), 321-640 the 32-lane one, longer ones the exact scalar kernel — bit-exact either way."""
+    MiSeq reads), 321-640 the 32-lane one, longer ones the striped kernel (k_sw_striped) — bit-exact either way."""
     gb, go = pkg.synth.random_genomes(3, 40_000, seed=8)
     rb, ro, _ = pkg.synth.paired_reads(gb, go, 300, read_len=read_len, seed=9, frag_mean=frag, frag_sd=30)
     res, tm = check_pipeline(pkg, gb, go, rb, ro, T.default_params(report_cigar=1))
@@ -423,6 +423,34 @@ def test_ssw_fast_domain_other_parameters(pkg, prm):
         tm = al.timings()
     check_overlaps(out, pool, want, wpool, fields=FIELDS[4:])
     assert tm["n_sw_slow"] == 0 and tm["n_sw_band"] > 3_000
+
+
+@pytest.mark.parametrize("prm", [(4, 4, 6, 2), (3, 5, 9, 3), (5, 6, 12, 3), (8, 9, 20, 5), (100, 100, 120, 60)])
+def test_ssw_fast_domain_beyond_the_packed_cells(pkg, prm):
+    """Parameters inside the plain-Gotoh domain that the packed kernels cannot hold (match > 3, mismatch > 4, or scores
+    beyond the 16-bit cells): every alignment runs the slow list (k_sw_striped). With match 100, 700-base reads score above
+    32767, where SSW's word pass saturates; the result is the saturated one, as the oracle computes it."""
+    m, x, go, ge = prm
+    if m == 100:
+        rng = np.random.default_rng(41)
+        ws = [pkg.synth.ACGT[rng.integers(0, 4, size=700)] for _ in range(300)]       # reads: the windows with 1 % substitutions
+        qs = [np.where(rng.random(700) < 0.01, pkg.synth.ACGT[rng.integers(0, 4, size=700)], w) for w in ws]
+        sets = [T.concat(qs) + T.concat(ws)]
+    else:
+        sets = [diverged_pairs(pkg, 3000, a, b, seed=950 + 7 * m + x + a) for a, b in ((150, 150), (120, 160))]
+    for q, qo, r, ro in sets:
+        n = len(qo) - 1
+        for cigar in (1, 0):
+            P = T.default_params(report_cigar=cigar, match=m, mismatch=x, gap_open=go, gap_extend=ge)
+            want, wpool = T.ko_ssw_batch(q, qo, r, ro, P, cigar_cap=64)
+            with pkg.Aligner(report_cigar=bool(cigar), max_cigar_ops=64, match=m, mismatch=x, gap_open=go, gap_extend=ge) as al:
+                assert al.fast
+                out, pool = al.ssw_batch(q, qo, r, ro)
+                tm = al.timings()
+            assert tm["n_sw_slow"] == n and tm["n_sw_fast"] == 0 and tm["n_sw_band"] == 0
+            if m == 100:
+                assert (want["sw_score"] == 32767).all() and not (want["flags"] & 1).any()
+            check_overlaps(out, pool, want, wpool, fields=FIELDS[4:], cigars=bool(cigar))
 
 
 @pytest.mark.parametrize("shape", [(150, 150), (120, 160)])
