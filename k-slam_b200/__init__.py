@@ -165,6 +165,9 @@ def lib():
     L.kslam_fetch_pairs_compact.argtypes = [vp, C.c_uint32, C.POINTER(_PairsCompact)]
     L.kslam_insert_size_limit_compact.argtypes = [vp, u64, C.c_uint32]
     L.kslam_insert_size_limit_compact.restype = C.c_uint32
+    L.kslam_insert_size_limit_counts.argtypes = [vp, C.c_uint32]
+    L.kslam_insert_size_limit_counts.restype = C.c_uint32
+    L.kslam_fetch_far_mates.argtypes = [vp, C.c_uint32, C.POINTER(u64), C.POINTER(vp)]
     L.kslam_batch_outputs_compact.argtypes = [C.POINTER(SamParams), C.POINTER(_SamDb), C.POINTER(_ReadBatch), C.POINTER(_PairsCompact), C.POINTER(C.c_uint32), vp, vp]
     L.kslam_comm_unique_id.argtypes = [vp]
     L.kslam_comm_init_rank.argtypes = [vp, C.c_uint32, C.c_uint32, vp, C.POINTER(vp)]
@@ -420,6 +423,14 @@ class Aligner:
         self._check(self.L.kslam_fetch_pairs_compact(self.h, threads, C.byref(out)), "kslam_fetch_pairs_compact")
         f = (lambda a: a.copy()) if copy else (lambda a: a)
         return f(_view(out.pairs, out.n_pairs, PAIR_COMPACT_DT)), int(out.insert_size_limit), f(_view(out.far, out.n_far, FAR_MATES_DT))
+
+    def fetch_far_mates(self, limit, copy=True):
+        """After pair_batch: the mates of every pair record with insert_size > limit, in pair order (kslam_fetch_far_mates;
+        what a caller needs once the insert-size limit of a run is known, e.g. after merging the batches of several GPUs)."""
+        n, ptr = C.c_uint64(), C.c_void_p()
+        self._check(self.L.kslam_fetch_far_mates(self.h, int(limit), C.byref(n), C.byref(ptr)), "kslam_fetch_far_mates")
+        far = _view(ptr.value, n.value, FAR_MATES_DT)
+        return far.copy() if copy else far
 
     def fetch_pairs(self, copy=True) -> "Pairs":
         """D2H of the last pair_batch(fetch=False)."""

@@ -243,15 +243,46 @@ void pair_overlaps(kslam_ctx *c) {
     CUDA_TRY(cudaStreamSynchronize(st));
     ns = (uint32_t)h_ns[0]; na = h_cnt[0];
   }
-  const uint32_t nbb = ns - na;
   c->n_sorted = ns;
   if (!ns) return;
   c->ov_sorted.reserve((size_t)ns * sizeof(kslam_overlap) + 64);
-  const uint32_t n_tiles = (ns + PM_TILE - 1) / PM_TILE;
-  k_pair_split<<<(n_tiles + 1 + 255) / 256, 256, 0, st>>>(c->ov.as<kslam_overlap>(), idx, na, nbb, mid, c->reads.max_len, n_tiles, tile_a);
-  k_pair_merge<<<n_tiles, PM_THREADS, 0, st>>>(c->ov.as<kslam_overlap>(), idx, na, nbb, mid, c->reads.max_len, tile_a,
-                                                c->ov_sorted.as<kslam_overlap>());
-  c->launches += 2;
+  const uint32_t bias = c->reads.max_len;
+  // the stable merge of the lists idx[0..la) and idx[la..la+lb) of `src` into dst[0..la+lb)
+  auto merge = [&](const kslam_overlap *src, const uint32_t *ix, uint32_t la, uint32_t lb, kslam_overlap *dst) {
+    const uint32_t tiles = (la + lb + PM_TILE - 1) / PM_TILE;
+    if (!tiles) return;
+    k_pair_split<<<(tiles + 1 + 255) / 256, 256, 0, st>>>(src, ix, la, lb, mid, bias, tiles, tile_a);
+    k_pair_merge<<<tiles, PM_THREADS, 0, st>>>(src, ix, la, lb, mid, bias, tile_a, dst);
+    c->launches += 2;
+  };
+  // An odd read count 2 mid + 1 (FASTQsequence.h:117-122 lets n2 = n1 + 1 through) gives the last read, 2 mid, pair id 0.
+  // Its passing overlaps are the tail [tail, ns) of the R2 list (the input is ordered by read), out of pair-id order, so the
+  // R2 list without that tail is merged with the R1 list first and the result then with the tail. The tail goes second:
+  // on equal keys the reference's order is by read index, and 2 mid is the largest.
+  uint32_t tail = ns;
+  if (c->reads.n & 1) {
+    k_pair_first_r2<<<1, 1, 0, st>>>(c->ov.as<kslam_overlap>(), n, 2 * mid, d_cnt + 1);   // first overlap of read 2 mid
+    c->launches++;
+    read_small(c, h_cnt + 1, d_cnt + 1, 4);
+    CUDA_TRY(cudaStreamSynchronize(st));
+    const uint32_t first = h_cnt[1];
+    if (idx == nullptr) tail = first;
+    else if (first < n) {                                  // passing overlaps before it: the exclusive scan's value there
+      read_small(c, h_cnt + 1, ppos + first, 4);
+      CUDA_TRY(cudaStreamSynchronize(st));
+      tail = h_cnt[1];
+    }
+  }
+  if (tail == ns) {
+    merge(c->ov.as<kslam_overlap>(), idx, na, ns - na, c->ov_sorted.as<kslam_overlap>());
+  } else {
+    c->pair_keys2.reserve((size_t)ns * sizeof(kslam_overlap) + 64);   // (used by nothing else)
+    kslam_overlap *tmp = c->pair_keys2.as<kslam_overlap>();
+    merge(c->ov.as<kslam_overlap>(), idx, na, tail - na, tmp);
+    // a one-list merge is a gather in list order: the tail's records follow the merged part in tmp
+    merge(idx ? c->ov.as<kslam_overlap>() : c->ov.as<kslam_overlap>() + tail, idx ? idx + tail : nullptr, ns - tail, 0, tmp + tail);
+    merge(tmp, nullptr, tail, ns - tail, c->ov_sorted.as<kslam_overlap>());
+  }
   const unsigned nbs = (ns + 255) / 256;
   c->pair_cnt.reserve((size_t)ns * 8 + 64);
   uint32_t *cnt = c->pair_cnt.as<uint32_t>(), *pos = cnt + ns;

@@ -495,6 +495,7 @@ static int cmp_pairsort(const void *a, const void *b) {
   if (x->entry != y->entry) return x->entry < y->entry ? -1 : 1;
   if (x->rel != y->rel) return x->rel < y->rel ? -1 : 1;
   if (x->read != y->read) return x->read < y->read ? -1 : 1;
+  if (x->rev_comp != y->rev_comp) return x->rev_comp < y->rev_comp ? -1 : 1;
   return 0;
 }
 void ko_sort_for_pairing(ko_overlap *ov, uint64_t n, uint32_t mid) {
